@@ -37,6 +37,32 @@ def test_reference_arm_other_ranks_do_nothing():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_caps_size_and_repeats_its_sample(tmp_path):
+    """--dump-outputs: float64 stays float64, other dtypes become float32, small outputs keep their shape, and an output
+    above its share of the 64 MB budget is written as a sample that is the same in every run."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    g = torch.Generator().manual_seed(3)
+    outs = {"loss": torch.tensor(2.5), "grad_a": torch.randn(256, 1000, generator=g).bfloat16(),
+            "grad_b": torch.randn(512, 197, 192, generator=g), "grad_c": torch.randn(7, generator=g).double()}
+    for d in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / d))
+    arrays = {f: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert sorted(arrays) == ["grad_a.npy", "grad_b.npy", "grad_c.npy", "loss.npy"]
+    assert sum(a.nbytes for a in arrays.values()) <= bench.DUMP_BYTES
+    assert arrays["loss.npy"].dtype == np.float32 and float(arrays["loss.npy"]) == 2.5
+    assert arrays["grad_a.npy"].shape == (256, 1000) and arrays["grad_a.npy"].dtype == np.float32
+    assert np.array_equal(arrays["grad_a.npy"], outs["grad_a"].float().numpy())
+    assert arrays["grad_c.npy"].dtype == np.float64 and np.array_equal(arrays["grad_c.npy"], outs["grad_c"].numpy())
+    b = arrays["grad_b.npy"]
+    assert b.ndim == 1 and 0 < b.size < outs["grad_b"].numel()
+    assert np.isin(b, outs["grad_b"].numpy()).all()
+    for f, a in arrays.items():
+        assert np.array_equal(a, np.load(tmp_path / "b" / f)), f
+
+
 def test_workload_registry_covers_the_baseline_configs():
     sys.path.insert(0, ROOT)
     import bench
