@@ -27,6 +27,29 @@ int check_launch(const char* what);  // cudaGetLastError -> DKD_E_LAUNCH
 
 constexpr int kNumSMs = 148;  // B200
 
+// ---- programmatic dependent launch ---------------------------------------------
+// A kernel launched by launch_pdl may start while its predecessor on the stream is still running (its CTAs are resident
+// and have called grid_dep_launch, or have exited), so launch latency and prologue overlap the predecessor's tail.  It
+// must call grid_dep_wait before its first global-memory access: the wait returns once the predecessor grid has
+// completed and its writes are visible.  Both are no-ops for a kernel launched without the attribute.
+__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+template <typename... KArgs, typename... Args>
+cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = 0;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
 // ---- element access ----------------------------------------------------------
 template <typename T> struct Elt;
 template <> struct Elt<float> {

@@ -11,6 +11,12 @@
 
 #include "common.cuh"
 
+// Phase stamps of the one-CTA-per-row kernel (point, value the stamp must wait for).  tools/probes/logit_phase_probe.cu
+// defines DKD_LOGIT_STAMP before including this file; the library compiles them to nothing.
+#ifndef DKD_LOGIT_STAMP
+#define DKD_LOGIT_STAMP(point, dep) ((void)0)
+#endif
+
 namespace dkd {
 namespace {
 
@@ -65,12 +71,13 @@ struct LogitKdParams {
 constexpr int kRuntimeMode = -2;
 constexpr float kL2e = 1.4426950408889634f;
 // gz_row / gzk_row: where this row's gradients go (global rows, or the ring stage of the streaming kernel; null = not
-// wanted).  PACK2: fp32-pair arithmetic in passes 2 and 3.
+// wanted).  PACK2: fp32-pair arithmetic in passes 2 and 3.  publish(base_row, kd_row) runs in every thread as soon as the
+// row's loss terms are known, before pass 3 writes the gradients.
 template <typename T, int VEC, int NV, int THREADS = kThreads, int LK = kRuntimeMode, int KK = kRuntimeMode,
-          bool PACK2 = (THREADS == kThreads)>
+          bool PACK2 = (THREADS == kThreads), typename Publish>
 __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, const T* z, const T* zk, const T* zt, const T* y,
                                           T* gz_row, T* gzk_row, float* scratch, int* s_arg, float* s_argv, float& base_out,
-                                          float& kd_out) {
+                                          float& kd_out, Publish&& publish) {
   const int64_t C = p.C;
   const int label_kind = LK == kRuntimeMode ? p.label_kind : LK;
   const int kd_kind = KK == kRuntimeMode ? p.kd_kind : KK;
@@ -144,7 +151,9 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
       pass1(it, rz[0], rk[0], rt[0]);
     }
   }
+  DKD_LOGIT_STAMP(1, mx[0]);   // loads landed
   block_max<3, THREADS>(mx, scratch);
+  DKD_LOGIT_STAMP(2, mx[0]);
   mx[1] *= invT;
   mx[2] *= invT;
   int64_t tgt = label;  // index whose one-hot enters the KD gradient (hard) -- label handled separately
@@ -271,6 +280,7 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
     t[1] = T2[1].x + T2[1].y;
   }
   block_sum<8, THREADS>(st8, scratch);
+  DKD_LOGIT_STAMP(3, s[0]);
   s[3] *= invT;
 
   // s[] >= 1 (the maximum contributes e^0): lg2.approx (absolute error 2^-22) and approximate reciprocals are exact
@@ -290,6 +300,7 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
     lse1 = mx[1] + __logf(s[1]);
     kd_row = lse1 - t[3];
   }
+  publish(base_row, kd_row);
 
   // ---- pass 3: gradients -----------------------------------------------------------------------
   const float wb = (kd_kind == 0 ? 1.f : 1.f - p.alpha) / Bf;           // d total / d base_row
@@ -363,30 +374,44 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
       }
     }
   }
+  DKD_LOGIT_STAMP(4, 0.f);   // gradient stores issued
 
   base_out = base_row;   // valid in every thread (block-wide sums); the caller stores or accumulates them
   kd_out = kd_row;
 }
 
-// Last CTA to finish folds the per-row partials in a fixed order (bit-reproducible) into {total, base, kd}.
-// `n_part`: number of partial sums in row_base / row_kd (one per row, or one per warp of the ring kernel)
+// The ticket: one add per CTA on a word of the workspace; the CTA that draws gridDim.x - 1 is the last one.  acq_rel: the
+// release publishes this thread's earlier stores (its CTA's partials) with the add, the acquire makes every partial
+// published before the adds that precede it visible to this thread (and, after a barrier, to its CTA).
+__device__ __forceinline__ unsigned int take_ticket(unsigned int* ticket) {
+  unsigned int old;
+  asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(old) : "l"(ticket) : "memory");
+  return old;
+}
+
+// The last CTA folds the per-row partials in a fixed order (bit-reproducible) into {total, base, kd} and resets the ticket.
+// `n_part`: number of partial sums in row_base / row_kd (one per row, or one per warp of the ring kernel).
+// Thread t adds rows t, t + THREADS, t + 2 * THREADS, ... in that order, then a fixed tree combines the threads.  The
+// loads of 8 rows per thread are all issued before the first add, so up to 8 * THREADS partials cost one L2 round trip.
 template <int THREADS = kThreads>
-__device__ __forceinline__ void logit_finalize(const LogitKdParams& p, float* scratch, bool* s_last, int64_t n_part) {
+__device__ __forceinline__ void logit_fold(const LogitKdParams& p, float* scratch, int64_t n_part) {
   const float Bf = (float)p.B, Cf = (float)p.C;
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned int done = atomicAdd(p.ticket, 1u);
-    *s_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!*s_last) return;
-  __threadfence();
   float acc[2] = {0.f, 0.f};
-  // fixed thread->row assignment and fixed tree => bit-reproducible
-  for (int64_t r = threadIdx.x; r < n_part; r += THREADS) {
-    acc[0] += __ldcg(p.row_base + r);
-    acc[1] += __ldcg(p.row_kd + r);
-  }
+  auto batch = [&](int64_t r0) {
+    float b[8], k[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      // a row past the end adds +0.f: acc is never -0.f (it starts at +0.f), so this gives the bits of skipping the add
+      const int64_t r = r0 + (int64_t)u * THREADS;
+      b[u] = r < n_part ? __ldcg(p.row_base + r) : 0.f;
+      k[u] = r < n_part ? __ldcg(p.row_kd + r) : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u) { acc[0] += b[u]; acc[1] += k[u]; }
+  };
+  batch(threadIdx.x);
+  for (int64_t r0 = threadIdx.x + 8 * THREADS; r0 < n_part; r0 += 8 * THREADS) batch(r0);
+  DKD_LOGIT_STAMP(6, acc[0]);
   block_sum<2, THREADS>(acc, scratch);
   if (threadIdx.x == 0) {
     const float base = acc[0] / Bf;  // 0 when label_kind < 0 (KD term only: total = alpha * kd)
@@ -397,7 +422,22 @@ __device__ __forceinline__ void logit_finalize(const LogitKdParams& p, float* sc
     p.loss_out[1] = base;
     p.loss_out[2] = kd;
     *p.ticket = 0u;  // ready for the next call on this workspace
+    DKD_LOGIT_STAMP(7, 0.f);
   }
+}
+
+// Ticket and fold for a kernel whose partials are final only at its end (the ring kernel's per-warp sums).
+template <int THREADS>
+__device__ __forceinline__ void logit_finalize(const LogitKdParams& p, float* scratch, bool* s_last, int64_t n_part) {
+  if (threadIdx.x == 0) {
+    __threadfence();
+    const unsigned int done = atomicAdd(p.ticket, 1u);
+    *s_last = (done == gridDim.x - 1);
+  }
+  __syncthreads();
+  if (!*s_last) return;
+  __threadfence();
+  logit_fold<THREADS>(p, scratch, n_part);
 }
 
 // fold by the first warp only (block size not known at compile time)
@@ -455,12 +495,23 @@ __global__ void __launch_bounds__(kFoldThreads) logit_fold_kernel(LogitKdParams 
   }
 }
 
+// TICKET: the last CTA folds the partials (otherwise logit_fold_kernel does, in a second launch).  Thread 0 publishes its
+// row's partials and takes the ticket as soon as block_sum has produced them; the add's round trip overlaps pass 3 and
+// the gradient stores, and its result is read only after them.  No fence waits for the gradient stores: nothing reads
+// them before the kernel ends.
+// Launched with programmatic dependent launch (launch_pdl).
 template <typename T, int VEC, int NV, int THREADS = kThreads, bool TICKET = true, int LK = kRuntimeMode, int KK = kRuntimeMode>
 __global__ void __launch_bounds__(THREADS) logit_kd_kernel(LogitKdParams p) {
   __shared__ float scratch[8 * (kThreads / 32)];
   __shared__ int s_arg[kThreads / 32];
   __shared__ float s_argv[kThreads / 32];
   __shared__ bool s_last;
+  DKD_LOGIT_STAMP(0, 0.f);
+  // The predecessor may still be running until the wait returns: the op that wrote the logits, or the previous call on
+  // this workspace (ticket, partials) and on gradient memory reused from it.
+  grid_dep_wait();
+  DKD_LOGIT_STAMP(8, 0.f);
+  grid_dep_launch();
   const int64_t row = blockIdx.x, C = p.C;
   const T* z = p.label_kind >= 0 ? reinterpret_cast<const T*>(p.z) + row * C : nullptr;
   const T* zk = p.kd_kind ? reinterpret_cast<const T*>(p.zk) + row * C : nullptr;
@@ -469,12 +520,23 @@ __global__ void __launch_bounds__(THREADS) logit_kd_kernel(LogitKdParams p) {
   T* gz = p.gz ? reinterpret_cast<T*>(p.gz) + row * C : nullptr;
   T* gzk = p.gzk ? reinterpret_cast<T*>(p.gzk) + row * C : nullptr;
   float base_row, kd_row;
-  logit_row<T, VEC, NV, THREADS, LK, KK>(p, row, z, zk, zt, y, gz, gzk, scratch, s_arg, s_argv, base_row, kd_row);
-  if (threadIdx.x == 0) {
-    p.row_base[row] = base_row;
-    p.row_kd[row] = kd_row;
+  unsigned int done = 0;
+  logit_row<T, VEC, NV, THREADS, LK, KK>(p, row, z, zk, zt, y, gz, gzk, scratch, s_arg, s_argv, base_row, kd_row,
+                                         [&](float base, float kd) {
+                                           if (threadIdx.x == 0) {
+                                             p.row_base[row] = base;
+                                             p.row_kd[row] = kd;
+                                             if (TICKET) done = take_ticket(p.ticket);
+                                           }
+                                         });
+  if (TICKET) {
+    if (threadIdx.x == 0) {
+      DKD_LOGIT_STAMP(5, (float)done);
+      s_last = (done == gridDim.x - 1);
+    }
+    __syncthreads();
+    if (s_last) logit_fold<THREADS>(p, scratch, p.B);
   }
-  if (TICKET) logit_finalize<THREADS>(p, scratch, &s_last, p.B);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -581,7 +643,7 @@ __global__ void __launch_bounds__(32 * kRingMaxWarps, 1) logit_ring_kernel(Logit
     float base_row, kd_row;
     logit_row<T, VEC, NV, 32, LK, KK, true>(p, row, LK >= 0 ? sz : nullptr, KK ? szk : nullptr, KK ? szt : nullptr, LK == 0 ? sy : nullptr,
                                             (p.gz && LK >= 0) ? sz : nullptr, (p.gzk && KK) ? szk : nullptr, nullptr, nullptr, nullptr,
-                                            base_row, kd_row);
+                                            base_row, kd_row, [](float, float) {});
     acc_base += base_row;   // this warp's rows, in row order: fixed for a given (B, grid)
     acc_kd += kd_row;
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the gradient rows (generic-proxy writes) -> visible to the bulk stores
@@ -616,9 +678,9 @@ __global__ void __launch_bounds__(32 * kRingMaxWarps, 1) logit_ring_kernel(Logit
 // one (threads, ticket) shape; NV by row length; the six usual (label_kind, kd_kind) modes are compiled in
 template <typename T, int VEC, int THREADS, bool TICKET, int LK, int KK>
 void launch_nv(const LogitKdParams& p, int64_t nchunk, dim3 grid, cudaStream_t stream) {
-  if (nchunk <= 1) logit_kd_kernel<T, VEC, 1, THREADS, TICKET, LK, KK><<<grid, THREADS, 0, stream>>>(p);
-  else if (nchunk <= 2) logit_kd_kernel<T, VEC, 2, THREADS, TICKET, LK, KK><<<grid, THREADS, 0, stream>>>(p);
-  else logit_kd_kernel<T, VEC, 4, THREADS, TICKET, LK, KK><<<grid, THREADS, 0, stream>>>(p);
+  if (nchunk <= 1) launch_pdl(logit_kd_kernel<T, VEC, 1, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
+  else if (nchunk <= 2) launch_pdl(logit_kd_kernel<T, VEC, 2, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
+  else launch_pdl(logit_kd_kernel<T, VEC, 4, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
 }
 template <typename T, int VEC, int THREADS, bool TICKET>
 void launch_mode(const LogitKdParams& p, int64_t nchunk, dim3 grid, cudaStream_t stream) {
@@ -686,7 +748,7 @@ int launch_logit_kd(const LogitKdParams& p, cudaStream_t stream) {
     return check_launch("dkd_logit_kd_fwdbwd: fold");
   }
   if (nchunk <= 4) launch_mode<T, VEC, kThreads, true>(p, nchunk, grid, stream);
-  else logit_kd_kernel<T, VEC, 0><<<grid, block, 0, stream>>>(p);
+  else launch_pdl(logit_kd_kernel<T, VEC, 0>, grid, block, stream, p);
   return check_launch("dkd_logit_kd_fwdbwd");
 }
 

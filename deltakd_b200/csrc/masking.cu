@@ -33,6 +33,10 @@ __global__ void mask_rank_kernel(const float* __restrict__ score, int L, int len
 template <typename T, int VEC>
 __global__ void scale_if_not_one_kernel(T* __restrict__ x, int64_t n_vec, T* __restrict__ x2, int64_t n_vec2,
                                         const float* __restrict__ scale) {
+  // launched with programmatic dependent launch: the predecessor (the op that wrote x / x2, or the one that wrote
+  // *scale) may still be running until the wait returns
+  grid_dep_wait();
+  grid_dep_launch();
   const float s = *scale;
   if (s == 1.0f) return;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -55,8 +59,8 @@ int launch_scale(void* x, int64_t n, void* x2, int64_t n2, const float* scale, c
   if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
   if (blocks < 1) blocks = 1;
   T *a = reinterpret_cast<T*>(x), *b = reinterpret_cast<T*>(x2);
-  if (vec_ok) scale_if_not_one_kernel<T, MAXV><<<(unsigned)blocks, 256, 0, st>>>(a, n_vec, b, n_vec2, scale);
-  else scale_if_not_one_kernel<T, 1><<<(unsigned)blocks, 256, 0, st>>>(a, n_vec, b, n_vec2, scale);
+  if (vec_ok) launch_pdl(scale_if_not_one_kernel<T, MAXV>, dim3((unsigned)blocks), dim3(256), st, a, n_vec, b, n_vec2, scale);
+  else launch_pdl(scale_if_not_one_kernel<T, 1>, dim3((unsigned)blocks), dim3(256), st, a, n_vec, b, n_vec2, scale);
   return check_launch("dkd_scale_if_not_one");
 }
 
