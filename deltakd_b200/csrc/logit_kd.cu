@@ -4,17 +4,20 @@
 //
 // One CTA per batch row.  The row of each operand is read from HBM exactly once (held in registers
 // when C <= THREADS*VEC*NV, otherwise re-read through L1/L2), max / log-sum-exp are block-reduced,
-// both gradient rows are written in the same launch, and the last CTA to finish folds the per-row
+// both gradient rows are written in the same launch, and a one-CTA launch behind it folds the per-row
 // partials in a fixed order (deterministic) into {total, base, kd}.
 // HBM-bound: algorithmic bytes = (reads + grad writes) * B * C * sizeof(elt); no tensor-core work.
 #include <stdlib.h>
 
 #include "common.cuh"
 
-// Phase stamps of the one-CTA-per-row kernel (point, value the stamp must wait for).  tools/probes/logit_phase_probe.cu
-// defines DKD_LOGIT_STAMP before including this file; the library compiles them to nothing.
+// Phase stamps (point, value the stamp must wait for) of the one-CTA-per-row kernel and of the fold.
+// tools/probes/logit_phase_probe.cu defines both before including this file; the library compiles them to nothing.
 #ifndef DKD_LOGIT_STAMP
 #define DKD_LOGIT_STAMP(point, dep) ((void)0)
+#endif
+#ifndef DKD_LOGIT_FOLD_STAMP
+#define DKD_LOGIT_FOLD_STAMP(point, dep) ((void)0)
 #endif
 
 namespace dkd {
@@ -380,16 +383,7 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
   kd_out = kd_row;
 }
 
-// The ticket: one add per CTA on a word of the workspace; the CTA that draws gridDim.x - 1 is the last one.  acq_rel: the
-// release publishes this thread's earlier stores (its CTA's partials) with the add, the acquire makes every partial
-// published before the adds that precede it visible to this thread (and, after a barrier, to its CTA).
-__device__ __forceinline__ unsigned int take_ticket(unsigned int* ticket) {
-  unsigned int old;
-  asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(old) : "l"(ticket) : "memory");
-  return old;
-}
-
-// The last CTA folds the per-row partials in a fixed order (bit-reproducible) into {total, base, kd} and resets the ticket.
+// One CTA folds the per-row partials in a fixed order (bit-reproducible) into {total, base, kd}.
 // `n_part`: number of partial sums in row_base / row_kd (one per row, or one per warp of the ring kernel).
 // Thread t adds rows t, t + THREADS, t + 2 * THREADS, ... in that order, then a fixed tree combines the threads.  The
 // loads of 8 rows per thread are all issued before the first add, so up to 8 * THREADS partials cost one L2 round trip.
@@ -411,7 +405,7 @@ __device__ __forceinline__ void logit_fold(const LogitKdParams& p, float* scratc
   };
   batch(threadIdx.x);
   for (int64_t r0 = threadIdx.x + 8 * THREADS; r0 < n_part; r0 += 8 * THREADS) batch(r0);
-  DKD_LOGIT_STAMP(6, acc[0]);
+  DKD_LOGIT_FOLD_STAMP(6, acc[0]);
   block_sum<2, THREADS>(acc, scratch);
   if (threadIdx.x == 0) {
     const float base = acc[0] / Bf;  // 0 when label_kind < 0 (KD term only: total = alpha * kd)
@@ -421,12 +415,12 @@ __device__ __forceinline__ void logit_fold(const LogitKdParams& p, float* scratc
     p.loss_out[0] = total;
     p.loss_out[1] = base;
     p.loss_out[2] = kd;
-    *p.ticket = 0u;  // ready for the next call on this workspace
-    DKD_LOGIT_STAMP(7, 0.f);
+    DKD_LOGIT_FOLD_STAMP(7, 0.f);
   }
 }
 
-// Ticket and fold for a kernel whose partials are final only at its end (the ring kernel's per-warp sums).
+// Ticket and fold for a kernel whose partials are final only at its end (the ring kernel's per-warp sums): one add per
+// CTA on a word of the workspace, and the CTA that draws gridDim.x - 1 folds and resets the word for the next call.
 template <int THREADS>
 __device__ __forceinline__ void logit_finalize(const LogitKdParams& p, float* scratch, bool* s_last, int64_t n_part) {
   if (threadIdx.x == 0) {
@@ -438,6 +432,7 @@ __device__ __forceinline__ void logit_finalize(const LogitKdParams& p, float* sc
   if (!*s_last) return;
   __threadfence();
   logit_fold<THREADS>(p, scratch, n_part);
+  if (threadIdx.x == 0) *p.ticket = 0u;
 }
 
 // fold by the first warp only (block size not known at compile time)
@@ -464,12 +459,27 @@ __device__ __forceinline__ void logit_finalize_any(const LogitKdParams& p, float
   }
 }
 
-// Large batches fold in a second launch: a 1024-thread CTA with 8 independent loads in flight per thread (a 128-thread
-// fold of 16 384 rows is ~130 dependent L2 round trips — it was most of the runtime of the fused form at B = 16 384).
+// The row kernel's partials are folded by a one-CTA launch right behind it (launch_pdl): its CTA is resident while the
+// rows run, and its dependency wait returns once every row CTA has exited and its partials are visible.  That grid
+// boundary is the whole inter-CTA protocol — no row CTA waits for another, and none pays a fence or an atomic.
+// Behind the 128-thread row kernel (B < 1024, or rows too long for the 2-warp one): kThreads threads, logit_fold's
+// thread -> row assignment and reduction tree.
+__global__ void __launch_bounds__(kThreads) logit_fold_small_kernel(LogitKdParams p) {
+  __shared__ float scratch[2 * (kThreads / 32)];
+  grid_dep_wait();
+  DKD_LOGIT_FOLD_STAMP(9, 0.f);
+  grid_dep_launch();
+  logit_fold<kThreads>(p, scratch, p.B);
+}
+
+// Large batches: a 1024-thread CTA with 8 independent loads in flight per thread (a 128-thread fold of 16 384 rows is
+// ~130 dependent L2 round trips — it was most of the runtime of the fused form at B = 16 384).
 // Fixed thread -> row assignment and fixed reduction tree: bit-reproducible.
 constexpr int kFoldThreads = 1024;
 __global__ void __launch_bounds__(kFoldThreads) logit_fold_kernel(LogitKdParams p) {
   __shared__ float scratch[2 * (kFoldThreads / 32)];
+  grid_dep_wait();
+  grid_dep_launch();
   float a0[8], a1[8];
 #pragma unroll
   for (int u = 0; u < 8; ++u) a0[u] = a1[u] = 0.f;
@@ -495,48 +505,57 @@ __global__ void __launch_bounds__(kFoldThreads) logit_fold_kernel(LogitKdParams 
   }
 }
 
-// TICKET: the last CTA folds the partials (otherwise logit_fold_kernel does, in a second launch).  Thread 0 publishes its
-// row's partials and takes the ticket as soon as block_sum has produced them; the add's round trip overlaps pass 3 and
-// the gradient stores, and its result is read only after them.  No fence waits for the gradient stores: nothing reads
-// them before the kernel ends.
-// Launched with programmatic dependent launch (launch_pdl).
-template <typename T, int VEC, int NV, int THREADS = kThreads, bool TICKET = true, int LK = kRuntimeMode, int KK = kRuntimeMode>
+// Asks L2 for `bytes` bytes at `src` without loading anything into the SM: one bulk prefetch when the range is 16-byte
+// aligned at both ends, otherwise one prefetch per 128-byte line spread over the CTA.  A hint only — it orders nothing
+// and returns no data.
+template <int THREADS>
+__device__ __forceinline__ void prefetch_l2(const void* src, int64_t bytes) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(src);
+  if (((a | (uintptr_t)bytes) & 15) == 0) {
+    const uint32_t n = (uint32_t)min(bytes, (int64_t)0xfffffff0);   // the size operand is 32-bit: a hint may stop short
+    if (threadIdx.x == 0) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(n) : "memory");
+  } else {
+    for (uintptr_t l = (a & ~(uintptr_t)127) + (uintptr_t)threadIdx.x * 128; l < a + (uintptr_t)bytes; l += THREADS * 128)
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(l));
+  }
+}
+
+// Thread 0 stores its row's partials as soon as block_sum has produced them; logit_fold_small_kernel or logit_fold_kernel
+// folds them in the next launch.  Launched with programmatic dependent launch (launch_pdl).
+template <typename T, int VEC, int NV, int THREADS = kThreads, int LK = kRuntimeMode, int KK = kRuntimeMode>
 __global__ void __launch_bounds__(THREADS) logit_kd_kernel(LogitKdParams p) {
   __shared__ float scratch[8 * (kThreads / 32)];
   __shared__ int s_arg[kThreads / 32];
   __shared__ float s_argv[kThreads / 32];
-  __shared__ bool s_last;
   DKD_LOGIT_STAMP(0, 0.f);
+  const int label_kind = LK == kRuntimeMode ? p.label_kind : LK;
+  const int kd_kind = KK == kRuntimeMode ? p.kd_kind : KK;
+  const int64_t row = blockIdx.x, C = p.C;
+  const T* z = label_kind >= 0 ? reinterpret_cast<const T*>(p.z) + row * C : nullptr;
+  const T* zk = kd_kind ? reinterpret_cast<const T*>(p.zk) + row * C : nullptr;
+  const T* zt = kd_kind ? reinterpret_cast<const T*>(p.zt) + row * C : nullptr;
+  const T* y = label_kind == 0 ? reinterpret_cast<const T*>(p.y) + row * C : nullptr;
+  T* gz = p.gz ? reinterpret_cast<T*>(p.gz) + row * C : nullptr;
+  T* gzk = p.gzk ? reinterpret_cast<T*>(p.gzk) + row * C : nullptr;
   // The predecessor may still be running until the wait returns: the op that wrote the logits, or the previous call on
-  // this workspace (ticket, partials) and on gradient memory reused from it.
+  // this workspace (partials) and on gradient memory reused from it.  Before the wait, the CTA only asks L2 for its
+  // operand rows, so that the loads after it find them there instead of in DRAM.  L2 is the GPU's point of coherence:
+  // stores of the predecessor that land after a prefetch update the prefetched lines, so no stale copy can be read.
+  const T* rows[4] = {z, zk, zt, y};
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+    if (rows[i]) prefetch_l2<THREADS>(rows[i], C * (int64_t)sizeof(T));
   grid_dep_wait();
   DKD_LOGIT_STAMP(8, 0.f);
   grid_dep_launch();
-  const int64_t row = blockIdx.x, C = p.C;
-  const T* z = p.label_kind >= 0 ? reinterpret_cast<const T*>(p.z) + row * C : nullptr;
-  const T* zk = p.kd_kind ? reinterpret_cast<const T*>(p.zk) + row * C : nullptr;
-  const T* zt = p.kd_kind ? reinterpret_cast<const T*>(p.zt) + row * C : nullptr;
-  const T* y = p.label_kind == 0 ? reinterpret_cast<const T*>(p.y) + row * C : nullptr;
-  T* gz = p.gz ? reinterpret_cast<T*>(p.gz) + row * C : nullptr;
-  T* gzk = p.gzk ? reinterpret_cast<T*>(p.gzk) + row * C : nullptr;
   float base_row, kd_row;
-  unsigned int done = 0;
   logit_row<T, VEC, NV, THREADS, LK, KK>(p, row, z, zk, zt, y, gz, gzk, scratch, s_arg, s_argv, base_row, kd_row,
                                          [&](float base, float kd) {
                                            if (threadIdx.x == 0) {
                                              p.row_base[row] = base;
                                              p.row_kd[row] = kd;
-                                             if (TICKET) done = take_ticket(p.ticket);
                                            }
                                          });
-  if (TICKET) {
-    if (threadIdx.x == 0) {
-      DKD_LOGIT_STAMP(5, (float)done);
-      s_last = (done == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (s_last) logit_fold<THREADS>(p, scratch, p.B);
-  }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -675,25 +694,25 @@ __global__ void __launch_bounds__(32 * kRingMaxWarps, 1) logit_ring_kernel(Logit
   else logit_finalize_any(p, scratch, &s_last, n_part);
 }
 
-// one (threads, ticket) shape; NV by row length; the six usual (label_kind, kd_kind) modes are compiled in
-template <typename T, int VEC, int THREADS, bool TICKET, int LK, int KK>
+// one block size; NV by row length; the six usual (label_kind, kd_kind) modes are compiled in
+template <typename T, int VEC, int THREADS, int LK, int KK>
 void launch_nv(const LogitKdParams& p, int64_t nchunk, dim3 grid, cudaStream_t stream) {
-  if (nchunk <= 1) launch_pdl(logit_kd_kernel<T, VEC, 1, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
-  else if (nchunk <= 2) launch_pdl(logit_kd_kernel<T, VEC, 2, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
-  else launch_pdl(logit_kd_kernel<T, VEC, 4, THREADS, TICKET, LK, KK>, grid, dim3(THREADS), stream, p);
+  if (nchunk <= 1) launch_pdl(logit_kd_kernel<T, VEC, 1, THREADS, LK, KK>, grid, dim3(THREADS), stream, p);
+  else if (nchunk <= 2) launch_pdl(logit_kd_kernel<T, VEC, 2, THREADS, LK, KK>, grid, dim3(THREADS), stream, p);
+  else launch_pdl(logit_kd_kernel<T, VEC, 4, THREADS, LK, KK>, grid, dim3(THREADS), stream, p);
 }
-template <typename T, int VEC, int THREADS, bool TICKET>
+template <typename T, int VEC, int THREADS>
 void launch_mode(const LogitKdParams& p, int64_t nchunk, dim3 grid, cudaStream_t stream) {
   if constexpr (VEC * sizeof(T) == 16) {   // specialise the vectorised kernels only
     const int lk = p.label_kind, kk = p.kd_kind;
-    if (lk == 0 && kk == 1) return launch_nv<T, VEC, THREADS, TICKET, 0, 1>(p, nchunk, grid, stream);
-    if (lk == 1 && kk == 1) return launch_nv<T, VEC, THREADS, TICKET, 1, 1>(p, nchunk, grid, stream);
-    if (lk == 0 && kk == 2) return launch_nv<T, VEC, THREADS, TICKET, 0, 2>(p, nchunk, grid, stream);
-    if (lk == 1 && kk == 2) return launch_nv<T, VEC, THREADS, TICKET, 1, 2>(p, nchunk, grid, stream);
-    if (lk == 0 && kk == 0) return launch_nv<T, VEC, THREADS, TICKET, 0, 0>(p, nchunk, grid, stream);
-    if (lk == 1 && kk == 0) return launch_nv<T, VEC, THREADS, TICKET, 1, 0>(p, nchunk, grid, stream);
+    if (lk == 0 && kk == 1) return launch_nv<T, VEC, THREADS, 0, 1>(p, nchunk, grid, stream);
+    if (lk == 1 && kk == 1) return launch_nv<T, VEC, THREADS, 1, 1>(p, nchunk, grid, stream);
+    if (lk == 0 && kk == 2) return launch_nv<T, VEC, THREADS, 0, 2>(p, nchunk, grid, stream);
+    if (lk == 1 && kk == 2) return launch_nv<T, VEC, THREADS, 1, 2>(p, nchunk, grid, stream);
+    if (lk == 0 && kk == 0) return launch_nv<T, VEC, THREADS, 0, 0>(p, nchunk, grid, stream);
+    if (lk == 1 && kk == 0) return launch_nv<T, VEC, THREADS, 1, 0>(p, nchunk, grid, stream);
   }
-  launch_nv<T, VEC, THREADS, TICKET, kRuntimeMode, kRuntimeMode>(p, nchunk, grid, stream);
+  launch_nv<T, VEC, THREADS, kRuntimeMode, kRuntimeMode>(p, nchunk, grid, stream);
 }
 
 // streaming launch for one compiled (label_kind, kd_kind) mode; false when the mode / shape is not covered
@@ -740,16 +759,19 @@ int launch_logit_kd(const LogitKdParams& p, cudaStream_t stream) {
       if (launch_ring<T, VEC, NV>(p, stream) == 0) return check_launch("dkd_logit_kd_fwdbwd: ring");
     }
   }
-  if (p.B >= 1024 && nchunk64 <= 4) {   // large batch: fold in a second launch
-    launch_mode<T, VEC, 64, false>(p, nchunk64, grid, stream);   // 2-warp CTAs (4-warp measured 3 % slower)
+  if (p.B >= 1024 && nchunk64 <= 4) {   // large batch: 2-warp CTAs (4-warp measured 3 % slower), 1024-thread fold
+    launch_mode<T, VEC, 64>(p, nchunk64, grid, stream);
     int rc = check_launch("dkd_logit_kd_fwdbwd");
     if (rc != DKD_OK) return rc;
-    logit_fold_kernel<<<1, kFoldThreads, 0, stream>>>(p);
+    launch_pdl(logit_fold_kernel, dim3(1), dim3(kFoldThreads), stream, p);
     return check_launch("dkd_logit_kd_fwdbwd: fold");
   }
-  if (nchunk <= 4) launch_mode<T, VEC, kThreads, true>(p, nchunk, grid, stream);
+  if (nchunk <= 4) launch_mode<T, VEC, kThreads>(p, nchunk, grid, stream);
   else launch_pdl(logit_kd_kernel<T, VEC, 0>, grid, block, stream, p);
-  return check_launch("dkd_logit_kd_fwdbwd");
+  int rc = check_launch("dkd_logit_kd_fwdbwd");
+  if (rc != DKD_OK) return rc;
+  launch_pdl(logit_fold_small_kernel, dim3(1), dim3(kThreads), stream, p);
+  return check_launch("dkd_logit_kd_fwdbwd: fold");
 }
 
 template <typename T>

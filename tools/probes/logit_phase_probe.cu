@@ -2,15 +2,18 @@
 // B = 256, C = 1000, bf16).  It compiles deltakd_b200/csrc/logit_kd.cu with DKD_LOGIT_STAMP defined: thread 0 of every CTA
 // records clock64 (SM cycles, comparable within a CTA) and %globaltimer (ns, comparable across CTAs) at
 //   0 kernel entry, 8 dependency resolved (after griddepcontrol.wait, where the kernel has one), 1 loads landed,
-//   2 block max done, 3 block sums done, 4 gradient stores issued, 5 ticket returned, 6 last CTA's fold loads summed,
-//   7 loss stored.
+//   2 block max done, 3 block sums done, 4 gradient stores issued, 5 ticket returned (builds whose last row CTA folds),
+//   9 fold kernel's dependency resolved (builds that fold in a launch of their own), 6 fold loads summed, 7 loss stored.
 // The workload is a CUDA graph of K calls on one stream and one workspace, inputs rotated through 97 sets (189 MiB > 126 MiB
-// of L2); each replay leaves the stamps of its last call, and R replays give R samples per CTA.  Times are reported from
-// the first CTA's start (entry, or dependency resolved) as the median CTA and as the last CTA (the one that folds).
+// of L2; K >= 97 so that a replay reads them all and the rows come from DRAM, as in bench.py); each replay leaves the
+// stamps of its last call, and R replays give R samples per CTA.  Times are reported from
+// the first row CTA's start (entry, or dependency resolved) as the median row CTA and as the last row CTA (the one whose
+// final stamp is latest: the folding CTA where a row CTA folds).  A fold kernel stamps a slot of its own; its points are
+// reported in both columns, its cycles counted from its dependency resolving.
 //
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 --expt-relaxed-constexpr -I deltakd_b200/csrc \
 //        -o build/logit_phase_probe tools/probes/logit_phase_probe.cu deltakd_b200/csrc/abi.cu
-//   build/logit_phase_probe [K=20] [R=200]
+//   build/logit_phase_probe [K=100] [R=200]
 // (-I another directory holding a stamped logit_kd.cu probes that version instead.)
 #include <algorithm>
 #include <cstdio>
@@ -20,23 +23,25 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
-constexpr int kPoints = 9;
+constexpr int kPoints = 10;
 constexpr int kMaxRows = 1024;
+constexpr int kFoldSlot = kMaxRows;
 struct Stamp {
   long long clk;
   unsigned long long ns;
 };
-__device__ Stamp g_stamp[kMaxRows][kPoints];
+__device__ Stamp g_stamp[kMaxRows + 1][kPoints];
 
-__device__ __forceinline__ void probe_stamp(int point, float dep) {
+__device__ __forceinline__ void probe_stamp(unsigned slot, int point, float dep) {
   asm volatile("" ::"f"(dep));   // the stamp is taken after `dep` is available
-  if (threadIdx.x == 0 && blockIdx.x < kMaxRows) {
+  if (threadIdx.x == 0 && slot <= kMaxRows) {
     unsigned long long ns;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    g_stamp[blockIdx.x][point] = {clock64(), ns};
+    g_stamp[slot][point] = {clock64(), ns};
   }
 }
-#define DKD_LOGIT_STAMP(point, dep) probe_stamp(point, dep)
+#define DKD_LOGIT_STAMP(point, dep) probe_stamp(blockIdx.x < kMaxRows ? blockIdx.x : ~0u, point, dep)
+#define DKD_LOGIT_FOLD_STAMP(point, dep) probe_stamp(kFoldSlot, point, dep)
 #include "logit_kd.cu"
 
 #define CK(x)                                                                          \
@@ -74,7 +79,7 @@ static double median(std::vector<double> v) {
 }
 
 int main(int argc, char** argv) {
-  const int K = argc > 1 ? atoi(argv[1]) : 20, R = argc > 2 ? atoi(argv[2]) : 200;
+  const int K = argc > 1 ? atoi(argv[1]) : 100, R = argc > 2 ? atoi(argv[2]) : 200;
   const int64_t B = 256, Cn = 1000, set_elems = 4 * B * Cn, nsets = 97;
   cudaDeviceProp prop;
   CK(cudaGetDeviceProperties(&prop, 0));
@@ -132,7 +137,7 @@ int main(int argc, char** argv) {
   // per point: samples of (median CTA) and (last CTA), ns from the first CTA's start; per phase: cycles
   std::vector<std::vector<double>> med_ns(kPoints), last_ns(kPoints), med_cyc(kPoints), last_cyc(kPoints);
   std::vector<double> mhz;
-  std::vector<Stamp> h(B * kPoints);
+  std::vector<Stamp> h((kMaxRows + 1) * kPoints);
   for (int r = 0; r < R; ++r) {
     CK(cudaEventRecord(e0, st));
     CK(cudaGraphLaunch(exec, st));
@@ -141,15 +146,22 @@ int main(int argc, char** argv) {
     float ms;
     CK(cudaEventElapsedTime(&ms, e0, e1));
     call_us.push_back(ms * 1e3 / K);
-    CK(cudaMemcpyFromSymbol(h.data(), g_stamp, B * kPoints * sizeof(Stamp)));
+    CK(cudaMemcpyFromSymbol(h.data(), g_stamp, h.size() * sizeof(Stamp)));
     auto at = [&](int cta, int pt) -> const Stamp& { return h[cta * kPoints + pt]; };
     auto start = [&](int cta) { return at(cta, 8).ns ? at(cta, 8) : at(cta, 0); };
     unsigned long long t0 = ~0ull;
     for (int c = 0; c < B; ++c) t0 = std::min(t0, start(c).ns);
+    auto final_pt = [&](int cta) {   // the CTA's latest stamp of this call
+      int f = -1;
+      for (int pt = 0; pt < kPoints; ++pt)
+        if (at(cta, pt).ns >= t0 && (f < 0 || at(cta, pt).ns > at(cta, f).ns)) f = pt;
+      return f;
+    };
     int last = -1;
     for (int c = 0; c < B; ++c)
-      if (at(c, 7).ns >= t0 && (last < 0 || at(c, 7).ns > at(last, 7).ns)) last = c;
-    if (last < 0) { fprintf(stderr, "no CTA stored the loss in replay %d\n", r); return 1; }
+      if (final_pt(c) >= 0 && (last < 0 || at(c, final_pt(c)).ns > at(last, final_pt(last)).ns)) last = c;
+    const bool fold_slot = at(kFoldSlot, 7).ns >= t0;
+    if (last < 0 || !(fold_slot || at(last, 7).ns >= t0)) { fprintf(stderr, "no CTA stored the loss in replay %d\n", r); return 1; }
     for (int pt = 0; pt < kPoints; ++pt) {
       std::vector<double> ns, cyc;
       for (int c = 0; c < B; ++c) {
@@ -162,13 +174,19 @@ int main(int argc, char** argv) {
         last_ns[pt].push_back((double)(at(last, pt).ns - t0));
         last_cyc[pt].push_back((double)(at(last, pt).clk - start(last).clk));
       }
+      if (fold_slot && at(kFoldSlot, pt).ns >= t0) {
+        const double fns = (double)(at(kFoldSlot, pt).ns - t0), fcyc = (double)(at(kFoldSlot, pt).clk - at(kFoldSlot, 9).clk);
+        med_ns[pt].push_back(fns); last_ns[pt].push_back(fns);
+        med_cyc[pt].push_back(fcyc); last_cyc[pt].push_back(fcyc);
+      }
     }
-    const double dns = (double)(at(last, 7).ns - at(last, 0).ns), dclk = (double)(at(last, 7).clk - at(last, 0).clk);
+    const int f = final_pt(last);
+    const double dns = (double)(at(last, f).ns - at(last, 0).ns), dclk = (double)(at(last, f).clk - at(last, 0).clk);
     if (dns > 0) mhz.push_back(dclk / dns * 1e3);
   }
   const char* names[kPoints] = {"entry", "loads landed", "block max", "block sums", "grad stores issued", "ticket returned",
-                                "fold loads summed", "loss stored", "dependency resolved"};
-  const int order[kPoints] = {0, 8, 1, 2, 3, 4, 5, 6, 7};
+                                "fold loads summed", "loss stored", "dependency resolved", "fold dependency resolved"};
+  const int order[kPoints] = {0, 8, 1, 2, 3, 4, 5, 9, 6, 7};
   printf("{\"device\": \"%s\", \"K\": %d, \"replays\": %d, \"call_us_median\": %.3f, \"globaltimer_step_ns\": "
          "{\"min\": %.0f, \"median\": %.0f}, \"sm_mhz_from_stamps\": %.0f, \"points\": [\n",
          prop.name, K, R, median(call_us), tdel.front(), median(tdel), median(mhz));
