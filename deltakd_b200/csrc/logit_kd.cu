@@ -74,8 +74,8 @@ struct LogitKdParams {
 constexpr int kRuntimeMode = -2;
 constexpr float kL2e = 1.4426950408889634f;
 // gz_row / gzk_row: where this row's gradients go (global rows, or the ring stage of the streaming kernel; null = not
-// wanted).  PACK2: fp32-pair arithmetic in passes 2 and 3.  publish(base_row, kd_row) runs in every thread as soon as the
-// row's loss terms are known, before pass 3 writes the gradients.
+// wanted).  PACK2: fp32-pair arithmetic in passes 2 and 3.  publish(base_row, kd_row) runs in every thread once the row's
+// loss terms are known, after pass 3 has issued the gradient stores.
 template <typename T, int VEC, int NV, int THREADS = kThreads, int LK = kRuntimeMode, int KK = kRuntimeMode,
           bool PACK2 = (THREADS == kThreads), typename Publish>
 __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, const T* z, const T* zk, const T* zt, const T* y,
@@ -294,16 +294,6 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
   if (label_kind < 0) base_row = 0.f;
   else if (label_kind == 0) base_row = lse0 * t[0] - t[1];
   else base_row = (1.f - p.smoothing) * (lse0 - (lam * t[2] + (1.f - lam) * t[0])) + p.smoothing * (lse0 - t[1] / Cf);
-  float lse1 = 0.f, lse2 = 0.f;
-  if (kd_kind == 1) {
-    lse1 = mx[1] + __logf(s[1]);
-    lse2 = mx[2] + __logf(s[2]);
-    kd_row = __fdividef(s[3], s[2]) - lse2 + lse1;  // sum_c p_t (log p_t - log p_s)
-  } else if (kd_kind == 2) {
-    lse1 = mx[1] + __logf(s[1]);
-    kd_row = lse1 - t[3];
-  }
-  publish(base_row, kd_row);
 
   // ---- pass 3: gradients -----------------------------------------------------------------------
   const float wb = (kd_kind == 0 ? 1.f : 1.f - p.alpha) / Bf;           // d total / d base_row
@@ -378,6 +368,21 @@ __device__ __forceinline__ void logit_row(const LogitKdParams& p, int64_t row, c
     }
   }
   DKD_LOGIT_STAMP(4, 0.f);   // gradient stores issued
+
+  // The KD term is formed after the gradient stores are issued: its latency overlaps their drain instead of delaying them.
+  if (kd_kind == 1) {
+    // sum_c p_t (log p_t - log p_s) = s3/s2 - lse2 + lse1, regrouped so that no term of size max/T enters the sum: with
+    // M1, M2 the shifts pass 2 subtracted in its exponents (log2 units, the same rounded values),
+    //   = s3/s2 + (M1 - M2) ln 2 + ln(s1/s2).
+    // Each term is O(|zt - zk| / T) and the row's KL is their small difference when the student is near the teacher.
+    // As lse1 - lse2, two O(max/T) values each rounded (and each off by the rounding of its own shift), the error was up
+    // to ~300 times the fp32 reference's at trained-logit scales.  __fmul_rn: the shifts are not contracted into FMAs.
+    const float M1 = __fmul_rn(mx[1], kL2e), M2 = __fmul_rn(mx[2], kL2e);
+    kd_row = fmaf(s[3], inv_s2, (M1 - M2) * 0.6931471805599453f) + log1pf((s[1] - s[2]) * inv_s2);
+  } else if (kd_kind == 2) {
+    kd_row = mx[1] + __logf(s[1]) - t[3];
+  }
+  publish(base_row, kd_row);
 
   base_out = base_row;   // valid in every thread (block-wide sums); the caller stores or accumulates them
   kd_out = kd_row;
@@ -520,8 +525,8 @@ __device__ __forceinline__ void prefetch_l2(const void* src, int64_t bytes) {
   }
 }
 
-// Thread 0 stores its row's partials as soon as block_sum has produced them; logit_fold_small_kernel or logit_fold_kernel
-// folds them in the next launch.  Launched with programmatic dependent launch (launch_pdl).
+// Thread 0 stores its row's partials after its gradient stores are issued; logit_fold_small_kernel or logit_fold_kernel
+// folds them in the next launch, whose dependency wait returns only once every row CTA has finished.  Launched with programmatic dependent launch (launch_pdl).
 template <typename T, int VEC, int NV, int THREADS = kThreads, int LK = kRuntimeMode, int KK = kRuntimeMode>
 __global__ void __launch_bounds__(THREADS) logit_kd_kernel(LogitKdParams p) {
   __shared__ float scratch[8 * (kThreads / 32)];
