@@ -5,14 +5,12 @@
 //
 // Launch sequence per layer (all on `stream`, no host sync):
 //   1. tokens_to_planes   s[B,Ts,Ds] (patch tokens only) -> bf16 planes S[P][M][Ds]      (P = 1 bf16 | 2 bf16x3)
-//   2. weight_to_planes   W[Dt,Ds] -> Wp[P][Dt][Ds] and its transpose Wt[P][Ds][Dt]
-//   3. gemm_tn + ResidualMse epilogue : Y = S W^T (tcgen05, TMEM) ; d = Y + b - t ; loss partial ; G = 2*scale*d
-//                                       written as bf16 planes G[P][M][Dt]            (teacher read in place)
-//   4. gemm_tn + StoreRows epilogue   : g_s[:,off:,:] = G W    (rows scattered into [B,Ts,Ds], CLS rows zeroed)
-//   5. gemm_nt (split-K, MN-major)    : g_W += G^T S, g_b += G^T 1 (ones-column trick)
-//   6. fold_partials                  : loss += sum of the per-CTA partials, fixed order (deterministic)
-#include <stdlib.h>
-
+//   2. weight_to_planes   W[Dt,Ds] -> Wp[P][Dt][Ds]   (step 3 reads it both K-major and MN-major: no transpose)
+//   3. align_fused_fwd_dgrad (one persistent tcgen05 kernel, align_fused.cuh):
+//        Y = S W^T ; d = Y + b - t ; loss partial ; G = 2*scale*d as bf16 planes G[P][M][Dt] (teacher read in place) ;
+//        g_s[:,off:,:] = G W    (rows scattered into [B,Ts,Ds], CLS rows zeroed)
+//   4. fold_partials      : loss += sum of the per-CTA partials, fixed order (deterministic)
+//   5. gemm_nt (split-K, MN-major, 3-CTA clusters) : g_W += G^T S, g_b += G^T 1 (ones-column trick)
 #include "align_fused.cuh"
 #include "align_ops.cuh"
 
@@ -21,14 +19,8 @@ namespace {
 
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-// DKD_ALIGN_FUSED = 0 keeps the three-launch form (forward, dgrad, wgrad) for A/B runs
-bool align_fused_enabled() {
-  static const bool on = [] { const char* e = getenv("DKD_ALIGN_FUSED"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 struct Workspace {
-  __nv_bfloat16 *S, *Wp, *Wt, *G, *ones;
+  __nv_bfloat16 *S, *Wp, *G, *ones;
   double* partials;
   size_t bytes;
 };
@@ -39,7 +31,6 @@ Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
   w.S = reinterpret_cast<__nv_bfloat16*>(take((size_t)P * M * Ds * 2));
   w.G = reinterpret_cast<__nv_bfloat16*>(take((size_t)P * M * Dt * 2));
   w.Wp = reinterpret_cast<__nv_bfloat16*>(take((size_t)P * Dt * Ds * 2));
-  w.Wt = reinterpret_cast<__nv_bfloat16*>(take((size_t)P * Dt * Ds * 2));
   w.ones = reinterpret_cast<__nv_bfloat16*>(take((size_t)2 * 64 * 64 * 2));
   w.partials = reinterpret_cast<double*>(take((size_t)kNumSMs * sizeof(double)));
   w.bytes = off;
@@ -75,47 +66,24 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   Workspace ws = carve(workspace, M, Ds, Dt, P);
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "dkd_align_mse_fwdbwd: workspace %zu < %zu", workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const bool want_grads = g_s != nullptr || g_W != nullptr || g_b != nullptr;
 
   // 1-2. operand planes
   rc = launch_tokens_to_planes(s, dtype, B, Ts, s_off, n_tok, Ds, P, nullptr, ws.S, st);
   if (rc != DKD_OK) return rc;
-  rc = launch_weight_to_planes(W, Dt, Ds, P, ws.Wp, want_grads ? ws.Wt : nullptr, st);
+  rc = launch_weight_to_planes(W, Dt, Ds, P, ws.Wp, nullptr, st);
   if (rc != DKD_OK) return rc;
 
-  // 3-4 fused: forward + residual + dgrad in one persistent kernel (align_fused.cuh); the G planes it leaves feed step 5
-  if (align_fused_enabled()) {
-    int grid = 0;
-    const char* what = "dkd_align_mse_fwdbwd: fused forward + dgrad";
-    rc = P == 2 ? align_fused_fwd_dgrad_t<2>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
-                                             g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what)
-                : align_fused_fwd_dgrad_t<1>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
-                                             g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what);
-    if (rc != DKD_OK) return rc;
-    rc = launch_fold_partials(ws.partials, grid, scale, loss, st);
-    if (rc != DKD_OK) return rc;
-    if (g_W || g_b) {
-      DKD_REQUIRE(g_W != nullptr, DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: g_b without g_W is not supported");
-      rc = align_wgrad(ws.G, ws.S, ws.ones, g_W, g_b, M, Ds, Dt, P, 1.f, st, "dkd_align_mse_fwdbwd: wgrad GEMM");
-      if (rc != DKD_OK) return rc;
-    }
-    return DKD_OK;
-  }
-
-  // 3. forward GEMM + residual epilogue
+  // 3. forward + residual + dgrad; the G planes it leaves feed step 5
   int grid = 0;
-  rc = align_forward_residual(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale, M, Ds, Dt, P,
-                              st, &grid, "dkd_align_mse_fwdbwd: forward GEMM");
+  const char* what = "dkd_align_mse_fwdbwd: fused forward + dgrad";
+  rc = P == 2 ? align_fused_fwd_dgrad_t<2>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
+                                           g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what)
+              : align_fused_fwd_dgrad_t<1>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
+                                           g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what);
   if (rc != DKD_OK) return rc;
+  // 4. loss
   rc = launch_fold_partials(ws.partials, grid, scale, loss, st);
   if (rc != DKD_OK) return rc;
-  if (!want_grads) return DKD_OK;
-
-  // 4. g_s = G W  (contract over Dt)
-  if (g_s) {
-    rc = align_dgrad(ws.G, ws.Wt, g_s, M, n_tok, Ts, s_off, Ds, Dt, P, dtype == DKD_BF16, 1.f, st, "dkd_align_mse_fwdbwd: dgrad GEMM");
-    if (rc != DKD_OK) return rc;
-  }
   // 5. g_W = G^T S, g_b = G^T 1
   if (g_W || g_b) {
     DKD_REQUIRE(g_W != nullptr, DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: g_b without g_W is not supported");

@@ -1,11 +1,9 @@
 // The three tcgen05 GEMMs around a Linear(Ds -> Dt) alignment head, shared by the losses that need the aligned
 // activations themselves (WassKD): forward rows, and the backward from a gradient-plane tensor G[P][M][Dt].
-//   align_forward_rows     : A[M, Dt] fp32 = S W^T + bias                 (gemm_tn, StoreRows epilogue)
-//   align_forward_residual : G = gscale (S W^T + bias - t), loss partials   (gemm_tn, ResidualMse epilogue)
+//   align_forward_rows : A[M, Dt] fp32 = S W^T + bias                 (gemm_tn, StoreRows epilogue)
 //   align_dgrad        : g_s[:, off:, :] = alpha * G W                (gemm_tn, rows scattered, special tokens zeroed)
-//   align_wgrad        : g_W = alpha * G^T S, g_b = alpha * G^T 1     (gemm_nt split-K, ones-column trick)
+//   align_wgrad        : g_W = alpha * G^T S, g_b = alpha * G^T 1     (gemm_nt split-K in 3-CTA clusters, ones-column trick)
 #pragma once
-#include <stdlib.h>
 #include "epilogues.cuh"
 #include "gemm_nt.cuh"
 #include "planes.cuh"
@@ -14,13 +12,11 @@ namespace dkd {
 
 using AlignCfg1 = GemmCfg<192, 1, 4, 2, 128, 1, 8>;   // one plane per stage (bf16 operands), 4-stage ring, 8 epilogue warps
 using AlignCfg2 = GemmCfg<192, 1, 2, 2, 128, 2, 8>;   // both planes per stage (bf16x3), 2 stages of 80 KB, 8 epilogue warps
-using AlignWgradCfg1 = GemmNtCfg<3, true, 208, 0, 4>;
+// wgrad: 3-CTA clusters (the three 128-wide teacher-channel tiles of one row split) with the S block multicast
+using AlignWgradCfg1 = GemmNtCfg<3, true, 208, 0, 4, 64, false, 1, 3>;
 // both planes per stage.  32 contraction rows per stage: 4 stages of 48 KB — with 64-row stages only two (96 KB each) fit and
 // every stage exposed a full TMA round trip (the kernel ran at 2.1 us per 64 rows against 0.65 us of MMA time)
-using AlignWgradCfg2 = GemmNtCfg<3, true, 208, 0, 4, 32, false, 2>;
-// ... as 3-CTA clusters (the three 128-wide teacher-channel tiles of one row split) with the S block multicast
-using AlignWgradCfg1C = GemmNtCfg<3, true, 208, 0, 4, 64, false, 1, 3>;
-using AlignWgradCfg2C = GemmNtCfg<3, true, 208, 0, 4, 32, false, 2, 3>;
+using AlignWgradCfg2 = GemmNtCfg<3, true, 208, 0, 4, 32, false, 2, 3>;
 
 template <class Cfg>
 inline int align_forward_rows_t(const __nv_bfloat16* S, const __nv_bfloat16* Wp, const float* bias, float* A, int64_t M, int Ds, int Dt,
@@ -40,32 +36,6 @@ inline int align_forward_rows_t(const __nv_bfloat16* S, const __nv_bfloat16* Wp,
   auto kern = gemm_tn_kernel<Cfg, L, E>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
   kern<<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(p);
-  return check_launch(what);
-}
-
-// d = S W^T + bias - t[:, t_off:] ; per-CTA loss partials ; G = gscale * d as planes (teacher read in place).
-// `grid_out` = number of partials written.
-template <class Cfg>
-inline int align_forward_residual_t(const __nv_bfloat16* S, const __nv_bfloat16* Wp, const float* bias, const void* t, int t_is_bf16,
-                                    int Tt, int t_off, int n_tok, __nv_bfloat16* G, double* partials, float gscale, int64_t M, int Ds,
-                                    int Dt, int P, cudaStream_t st, int* grid_out, const char* what) {
-  using L = PlaneLoader<Cfg>;
-  using E = ResidualMseEpi<Cfg>;
-  GemmParams<L, E> p;
-  int rc = make_plane_tmap(&p.ld.tmA, S, P, M, Ds, Ds, M * Ds, Cfg::BM, what);
-  if (rc != DKD_OK) return rc;
-  rc = make_plane_tmap(&p.ld.tmB, Wp, P, Dt, Ds, Ds, (int64_t)Dt * Ds, Cfg::BN, what);
-  if (rc != DKD_OK) return rc;
-  p.ld.k_blocks = Ds / 64; p.ld.nterms = P == 2 ? 3 : 1;
-  p.ep.t = t; p.ep.bias = bias; p.ep.G = G; p.ep.partials = partials;
-  p.ep.M = M; p.ep.N = Dt; p.ep.n_tok = n_tok; p.ep.Tt = Tt; p.ep.t_off = t_off; p.ep.planes = P;
-  p.ep.gscale = gscale; p.ep.t_is_bf16 = t_is_bf16;
-  p.m_tiles = (int)((M + Cfg::BM - 1) / Cfg::BM); p.n_tiles = Dt / Cfg::BN;
-  const int grid = min(kNumSMs, p.m_tiles * p.n_tiles);
-  auto kern = gemm_tn_kernel<Cfg, L, E>;
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
-  kern<<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(p);
-  *grid_out = grid;
   return check_launch(what);
 }
 
@@ -96,14 +66,6 @@ inline int align_forward_rows(const __nv_bfloat16* S, const __nv_bfloat16* Wp, c
   return P == 2 ? align_forward_rows_t<AlignCfg2>(S, Wp, bias, A, M, Ds, Dt, P, st, what)
                 : align_forward_rows_t<AlignCfg1>(S, Wp, bias, A, M, Ds, Dt, P, st, what);
 }
-inline int align_forward_residual(const __nv_bfloat16* S, const __nv_bfloat16* Wp, const float* bias, const void* t, int t_is_bf16,
-                                  int Tt, int t_off, int n_tok, __nv_bfloat16* G, double* partials, float gscale, int64_t M, int Ds,
-                                  int Dt, int P, cudaStream_t st, int* grid_out, const char* what) {
-  return P == 2 ? align_forward_residual_t<AlignCfg2>(S, Wp, bias, t, t_is_bf16, Tt, t_off, n_tok, G, partials, gscale, M, Ds, Dt, P, st,
-                                                      grid_out, what)
-                : align_forward_residual_t<AlignCfg1>(S, Wp, bias, t, t_is_bf16, Tt, t_off, n_tok, G, partials, gscale, M, Ds, Dt, P, st,
-                                                      grid_out, what);
-}
 // g_lo_zero: the lo plane of G is identically zero and is neither read nor multiplied (WassKD's +-1 gradient plane)
 inline int align_dgrad(const __nv_bfloat16* G, const __nv_bfloat16* Wt, void* g_s, int64_t M, int n_tok, int Ts, int s_off, int Ds, int Dt,
                        int P, int out_is_bf16, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
@@ -131,32 +93,18 @@ inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bf
   p.ld.total_row_blocks = (int)((M + Cfg::KROWS - 1) / Cfg::KROWS);
   p.nterms = P == 2 ? 3 : 1;
   p.a_lo_zero = (Cfg::PLANES == 2 && g_lo_zero) ? 1 : 0;
-  if constexpr (Cfg::CLUSTER > 1) {
-    static const int resident = [] {
-      auto kern = gemm_nt_kernel<Cfg, L>;
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
-      return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
-    }();
-    nt_make_splits(p.ld.total_row_blocks, resident, &p.ld.splits, &p.ld.row_blocks_per_split);
-    launch_gemm_nt<Cfg, L>(p, min(resident, p.ld.splits) * Cfg::CLUSTER, st);
-  } else {
-    nt_make_splits(p.ld.total_row_blocks, kNumSMs / p.ld.na_tiles, &p.ld.splits, &p.ld.row_blocks_per_split);
-    launch_gemm_nt<Cfg, L>(p, min(kNumSMs, p.ld.na_tiles * p.ld.splits), st);
-  }
+  static const int resident = [] {
+    auto kern = gemm_nt_kernel<Cfg, L>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
+    return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
+  }();
+  nt_make_splits(p.ld.total_row_blocks, resident, &p.ld.splits, &p.ld.row_blocks_per_split);
+  launch_gemm_nt<Cfg, L>(p, min(resident, p.ld.splits) * Cfg::CLUSTER, st);
   return check_launch(what);
-}
-
-// DKD_ALIGN_WGRAD_CLUSTER = 1 | 3
-inline int align_wgrad_cluster() {
-  static const int v = [] { const char* e = getenv("DKD_ALIGN_WGRAD_CLUSTER"); const int x = e ? atoi(e) : 3; return x == 1 ? 1 : 3; }();
-  return v;
 }
 
 inline int align_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bfloat16* ones, float* g_W, float* g_b, int64_t M, int Ds, int Dt,
                        int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
-  if (align_wgrad_cluster() == 3 && Dt == 384)
-    return P == 2 ? align_wgrad_t<AlignWgradCfg2C>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
-                  : align_wgrad_t<AlignWgradCfg1C>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
   return P == 2 ? align_wgrad_t<AlignWgradCfg2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
                 : align_wgrad_t<AlignWgradCfg1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
 }

@@ -36,25 +36,9 @@ struct ConvRowsLoader {
     sm100::tma_prefetch_desc(&p.tmX);
     sm100::tma_prefetch_desc(&p.tmW);
   }
-  static __device__ __forceinline__ void issue(const Params& p, int kit, int mt, int nt, uint8_t* sA, uint8_t* sB, uint64_t* bar) {
-    const int term = kit / KB, r = kit - term * KB;
-    const int tap = r / 6, cb = r - tap * 6;
-    const int dy = tap / 3, dx = tap - dy * 3;
-    int pa, pb;
-    term_planes(term, p.nterms, pa, pb);
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) {
-      const int hb = mt * ROWS + rr;
-      const int sh = hb % kHW + dy - 1;
-      const bool ok = sh >= 0 && sh < kHW && hb < p.total_hrows;
-      sm100::tma_load_4d(sA + rr * kRowBytes, &p.tmX, bar, cb * 64, dx - 1, ok ? hb + dy - 1 : -4, pa);
-    }
-    sm100::tma_load_3d(sB, &p.tmW, bar, tap * 384 + cb * 64, nt * Cfg::BN, pb);
-    sm100::tma_load_3d(sB + 192 * 128, &p.tmW, bar, tap * 384 + cb * 64, nt * Cfg::BN + 192, pb);
-  }
-  // Cluster form: the CTAs of a cluster work on different image rows but need the SAME 384 x 64 weight block at every K
-  // iteration — CTA `crank` fetches rows [crank * 384/CL, ...) of it and multicasts them to the whole cluster (tmW's box
-  // has 384 / CLUSTER rows).  Weight traffic L2 -> SM drops from 48 KB to 48/CL KB per K block and CTA.
+  // The CTAs of a cluster work on different image rows but need the SAME 384 x 64 weight block at every K iteration —
+  // CTA `crank` fetches rows [crank * 384/CL, ...) of it and multicasts them to the whole cluster (tmW's box has
+  // 384 / CLUSTER rows).  Weight traffic L2 -> SM drops from 48 KB to 48/CL KB per K block and CTA.
   static constexpr int W_ROWS = 384 / Cfg::CLUSTER;
   static __device__ __forceinline__ void issue_cluster(const Params& p, int kit, int mt, int nt, uint8_t* sA, uint8_t* sB, uint64_t* bar,
                                                        int crank) {
@@ -164,29 +148,16 @@ template <class Cfg>
 struct NtConvLoader {
   using Params = NtConvParams;
   using Item = NtItem;
-  static constexpr int COMBOS = 9 * 3 * 2;   // tap x co tile (128) x ci half (192)
-  static constexpr int COMBOS_CLUSTER = 9 * 2;
+  static constexpr int COMBOS_CLUSTER = 9 * 2;   // tap x ci half (192); the cluster's 3 CTAs are the co tiles (128)
   static constexpr uint32_t TX_BYTES = Cfg::STAGE_BYTES;
   static_assert(Cfg::KROWS == 8 * kHW && Cfg::NB_BOXES == 3 && !Cfg::ONES, "conv wgrad stage = 8 image rows x 192 channels");
-  static_assert(Cfg::CLUSTER == 1 || Cfg::CLUSTER == 3, "cluster form = the 3 output-channel tiles");
-  static __device__ __forceinline__ int num_items(const Params& p) { return (Cfg::CLUSTER > 1 ? COMBOS_CLUSTER : COMBOS) * p.splits; }
+  static_assert(Cfg::CLUSTER == 3, "a cluster = the 3 output-channel tiles");
+  static __device__ __forceinline__ int num_items(const Params& p) { return COMBOS_CLUSTER * p.splits; }
   static __device__ __forceinline__ void prefetch(const Params& p) {
     sm100::tma_prefetch_desc(&p.tmG);
     sm100::tma_prefetch_desc(&p.tmX);
   }
-  static __device__ __forceinline__ void decode(const Params& p, int item, Item& it) {
-    const int combo = item % COMBOS, split = item / COMBOS;
-    const int tap = combo / 6, rem = combo - tap * 6;
-    const int co_tile = rem >> 1, ci_half = rem & 1;
-    it.rb0 = split * p.row_blocks_per_split;
-    it.rb1 = min(it.rb0 + p.row_blocks_per_split, p.total_row_blocks);
-    it.a_col0 = co_tile * 128;
-    it.b_col0 = ci_half * 192;
-    it.d_off = ((int64_t)tap * 384 + co_tile * 128) * 384 + ci_half * 192;   // dWt[tap][co][ci]
-    it.dcol_off = -1;
-    it.aux = tap;
-  }
-  // ---- cluster form (3 CTAs = the 3 output-channel tiles of one (tap, ci half, row split)): same shifted X rows for all
+  // A cluster's 3 CTAs are the 3 output-channel tiles of one (tap, ci half, row split): same shifted X rows for all
   // three, so CTA `crank` fetches channel box `crank` of every image row and multicasts it: per 16-row K step a CTA pulls
   // 4 KB (its G tile) + 2 KB from L2 instead of 4 + 6 KB.
   static __device__ __forceinline__ int num_items_cluster(const Params& p) { return COMBOS_CLUSTER * p.splits; }
@@ -216,23 +187,6 @@ struct NtConvLoader {
       const int coord = ok ? hb + dy - 1 : -4;
       sm100::tma_load_4d_mc(b + (size_t)crank * Cfg::BOX_BYTES + rr * kRowBytes, &p.tmX, bar, it.b_col0 + crank * 64, dx - 1, coord, pb,
                             (uint16_t)0x7);
-    }
-  }
-  static __device__ __forceinline__ void issue(const Params& p, const Item& it, int term, int nterms, int rb, uint8_t* a, uint8_t* b, uint64_t* bar) {
-    int pa, pb;
-    term_planes(term, nterms, pa, pb);
-    const int dy = it.aux / 3, dx = it.aux - dy * 3;
-    sm100::tma_load_3d(a, &p.tmG, bar, it.a_col0, rb * Cfg::KROWS, pa);
-    sm100::tma_load_3d(a + Cfg::BOX_BYTES, &p.tmG, bar, it.a_col0 + 64, rb * Cfg::KROWS, pa);
-#pragma unroll
-    for (int rr = 0; rr < 8; ++rr) {
-      const int hb = rb * 8 + rr;
-      const int sh = hb % kHW + dy - 1;
-      const bool ok = sh >= 0 && sh < kHW && hb < p.total_hrows;
-      const int coord = ok ? hb + dy - 1 : -4;
-#pragma unroll
-      for (int i = 0; i < 3; ++i)
-        sm100::tma_load_4d(b + (size_t)i * Cfg::BOX_BYTES + rr * kRowBytes, &p.tmX, bar, it.b_col0 + i * 64, dx - 1, coord, pb);
     }
   }
 };

@@ -7,8 +7,6 @@
 // both gradient rows are written in the same launch, and a one-CTA launch behind it folds the per-row
 // partials in a fixed order (deterministic) into {total, base, kd}.
 // HBM-bound: algorithmic bytes = (reads + grad writes) * B * C * sizeof(elt); no tensor-core work.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 // Phase stamps (point, value the stamp must wait for) of the one-CTA-per-row kernel and of the fold.
@@ -747,10 +745,6 @@ int launch_ring(const LogitKdParams& p, cudaStream_t stream) {
   if (lk == 1 && kk == 0) return launch_ring_mode<T, VEC, NV, 1, 0>(p, stream);
   return 1;
 }
-bool ring_enabled() {
-  static const bool on = [] { const char* e = getenv("DKD_LOGIT_RING"); return !(e && e[0] == '0'); }();
-  return on;
-}
 
 template <typename T, int VEC>
 int launch_logit_kd(const LogitKdParams& p, cudaStream_t stream) {
@@ -760,7 +754,7 @@ int launch_logit_kd(const LogitKdParams& p, cudaStream_t stream) {
   const int64_t nchunk64 = (p.C + 64 * VEC - 1) / (64 * VEC);
   if constexpr (VEC * sizeof(T) == 16) {   // large batch, 16-byte aligned rows of 1-4 KB: persistent bulk-copy ring
     constexpr int NV = 32 / VEC;           // 32 elements per lane and operand: C <= 1024
-    if (p.B >= 1024 && p.C * (int64_t)sizeof(T) >= 1024 && p.C <= 32 * VEC * NV && ring_enabled()) {
+    if (p.B >= 1024 && p.C * (int64_t)sizeof(T) >= 1024 && p.C <= 32 * VEC * NV) {
       if (launch_ring<T, VEC, NV>(p, stream) == 0) return check_launch("dkd_logit_kd_fwdbwd: ring");
     }
   }

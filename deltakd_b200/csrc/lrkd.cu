@@ -597,8 +597,6 @@ __global__ void __launch_bounds__(32 * kCW, 1) jacobi_cluster_kernel(JacobiParam
 // host: can a 16-CTA cluster of this kernel be scheduled on this device?  (non-portable cluster size; cached)
 bool jacobi_cluster_available() {
   static const bool ok = [] {
-    const char* env = getenv("DKD_LRKD_CLUSTER");
-    if (env && env[0] == '0') return false;
     if (cudaFuncSetAttribute(jacobi_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess ||
         cudaFuncSetAttribute(jacobi_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem) != cudaSuccess) {
       cudaGetLastError();

@@ -14,8 +14,6 @@
 //   bwd : conv2 wgrad (G^T (*) H) + colsum(G) ; conv2 dgrad (dReLU epilogue) -> DH ; conv1 wgrad + colsum(DH) ;
 //         conv1 dgrad -> dXm (into G) ; masked colsum(dXm) -> g_b_align, g_mask_token ;
 //         g_s = (1-mask) * dXm W_align (row-masked store) ; g_W_align = dXm^T S'
-#include <stdlib.h>
-
 #include "conv.cuh"
 #include "planes.cuh"
 
@@ -23,12 +21,11 @@ namespace dkd {
 namespace {
 
 using AlignCfg = GemmCfg<192, 1, 4, 2, 128, 1, 8>;   // X tile 128 x 192 (K = 192), 8 epilogue warps
-using ConvCfg = GemmCfg<384, 2, 3, 1, 126, 1, 8>;    // 9 image rows x 384 channels, K = 9 x 384, 8 epilogue warps
-using ConvCfgC2 = GemmCfg<384, 2, 3, 1, 126, 1, 8, 2>;   // ... as clusters of 2 / 4 CTAs with the weight block multicast
-using ConvCfgC4 = GemmCfg<384, 2, 3, 1, 126, 1, 8, 4>;
+// 9 image rows x 384 channels, K = 9 x 384, 8 epilogue warps; clusters of 2 CTAs with the weight block multicast
+using ConvCfg = GemmCfg<384, 2, 3, 1, 126, 1, 8, 2>;
 using DalignCfg = GemmCfg<192, 1, 4, 2, 128, 1, 8>;  // g_s tile 128 x 192 (K = 384)
-using ConvWgradCfg = GemmNtCfg<3, false, 192, 0, 3, 112>;  // dW tile 128(co) x 192(ci), 8 image rows per stage
-using ConvWgradCfgC3 = GemmNtCfg<3, false, 192, 0, 3, 112, false, 1, 3>;   // ... 3-CTA clusters, shifted-X block multicast
+// dW tile 128(co) x 192(ci), 8 image rows per stage; 3-CTA clusters with the shifted-X block multicast
+using ConvWgradCfg = GemmNtCfg<3, false, 192, 0, 3, 112, false, 1, 3>;
 using AlignWgradCfg = GemmNtCfg<3, false, 192, 0, 4>;      // g_W_align tile 128 x 192
 
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -70,22 +67,17 @@ int launch_tn(GemmParams<L, E>& p, cudaStream_t st, const char* what, int* grid_
   return check_launch(what);
 }
 
-// DKD_CONV_CLUSTER = 1 | 2 | 4: CTAs per cluster of the generator convolutions (weight block multicast)
-int conv_cluster() {
-  static const int v = [] { const char* e = getenv("DKD_CONV_CLUSTER"); const int x = e ? atoi(e) : 2; return (x == 1 || x == 2 || x == 4) ? x : 2; }();
-  return v;
-}
-
 // one generator convolution (forward or dgrad): out planes = epilogue(conv3x3(in planes; w planes))
-template <int MODE, class Cfg>
-int run_conv_t(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParams ep, int64_t B, int C, int P, cudaStream_t st,
-               const char* what, int* grid_out) {
+template <int MODE>
+int run_conv(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParams ep, int64_t B, int C, int P, cudaStream_t st,
+             const char* what, int* grid_out = nullptr) {
+  using Cfg = ConvCfg;
   using L = ConvRowsLoader<Cfg>;
   using E = ConvEpi<Cfg, MODE>;
   GemmParams<L, E> p;
   int rc = make_image_tmap(&p.ld.tmX, in, B, C, P, what);
   if (rc != DKD_OK) return rc;
-  rc = make_plane_tmap(&p.ld.tmW, wplanes, P, C, 9 * C, 9 * C, (int64_t)C * 9 * C, Cfg::CLUSTER > 1 ? 384 / Cfg::CLUSTER : 192, what);
+  rc = make_plane_tmap(&p.ld.tmW, wplanes, P, C, 9 * C, 9 * C, (int64_t)C * 9 * C, L::W_ROWS, what);
   if (rc != DKD_OK) return rc;
   p.ld.total_hrows = (int)(B * kHW);
   p.ld.nterms = P == 2 ? 3 : 1;
@@ -94,26 +86,11 @@ int run_conv_t(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiPar
   p.n_tiles = 1;
   return launch_tn<Cfg, L, E>(p, st, what, grid_out);
 }
-template <int MODE>
-int run_conv(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParams ep, int64_t B, int C, int P, cudaStream_t st,
-             const char* what, int* grid_out = nullptr) {
-  switch (conv_cluster()) {
-    case 4: return run_conv_t<MODE, ConvCfgC4>(in, wplanes, ep, B, C, P, st, what, grid_out);
-    case 2: return run_conv_t<MODE, ConvCfgC2>(in, wplanes, ep, B, C, P, st, what, grid_out);
-    default: return run_conv_t<MODE, ConvCfg>(in, wplanes, ep, B, C, P, st, what, grid_out);
-  }
-}
-
-// DKD_WGRAD_CLUSTER = 1 | 3: CTAs per cluster of the conv weight-gradient GEMMs
-int wgrad_cluster() {
-  static const int v = [] { const char* e = getenv("DKD_WGRAD_CLUSTER"); const int x = e ? atoi(e) : 3; return x == 1 ? 1 : 3; }();
-  return v;
-}
 
 // dWt[tap][co][ci] = sum_m G[m, co] * X[m + shift(tap), ci]
-template <class Cfg>
-int run_conv_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, int64_t B, int64_t M, int C, int P, cudaStream_t st,
-                     const char* what) {
+int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, int64_t B, int64_t M, int C, int P, cudaStream_t st,
+                   const char* what) {
+  using Cfg = ConvWgradCfg;
   using L = NtConvLoader<Cfg>;
   GemmNtParamsT<Cfg, L> p;
   int rc = make_plane_tmap(&p.ld.tmG, G, P, M, C, C, M * C, Cfg::KROWS, what);
@@ -122,32 +99,22 @@ int run_conv_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt,
   if (rc != DKD_OK) return rc;
   p.ld.total_hrows = (int)(B * kHW);
   p.ld.total_row_blocks = (p.ld.total_hrows + 7) / 8;
-  // Items = (tap, co tile, ci half) x row splits over the CTAs (cluster form: (tap, ci half) x splits over the clusters).
-  // The split count is chosen so that the items fill whole waves: the former fixed 6 splits gave 324 items on 148 CTAs
-  // = 2.19 waves, i.e. a makespan of 3 waves for 2.19 waves of work (27 % idle).
-  const int combos = Cfg::CLUSTER > 1 ? L::COMBOS_CLUSTER : L::COMBOS;
-  int slots = kNumSMs;
-  if constexpr (Cfg::CLUSTER > 1) {
-    static const int resident = [] {
-      auto kern = gemm_nt_kernel<Cfg, L>;
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
-      return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
-    }();
-    slots = resident;
-  }
-  const int sp = nt_best_splits(combos, slots, p.ld.total_row_blocks, 4, 16);
+  // Items = (tap, ci half) x row splits over the clusters.  The split count is chosen so that the items fill whole waves:
+  // the former fixed 6 splits gave 324 items on 148 CTAs = 2.19 waves, i.e. a makespan of 3 waves for 2.19 waves of work
+  // (27 % idle).
+  static const int resident = [] {
+    auto kern = gemm_nt_kernel<Cfg, L>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
+    return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
+  }();
+  const int sp = nt_best_splits(L::COMBOS_CLUSTER, resident, p.ld.total_row_blocks, 4, 16);
   nt_make_splits(p.ld.total_row_blocks, sp, &p.ld.splits, &p.ld.row_blocks_per_split);
   p.ep.D = dWt; p.ep.Dcol = nullptr; p.ep.ldd = C; p.ep.alpha = 1.f;
   p.nterms = P == 2 ? 3 : 1;
   cudaMemsetAsync(dWt, 0, (size_t)9 * C * C * sizeof(float), st);
-  int grid = min(slots, combos * p.ld.splits) * Cfg::CLUSTER;
+  int grid = min(resident, L::COMBOS_CLUSTER * p.ld.splits) * Cfg::CLUSTER;
   launch_gemm_nt<Cfg, L>(p, grid, st);
   return check_launch(what);
-}
-int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, int64_t B, int64_t M, int C, int P, cudaStream_t st,
-                   const char* what) {
-  return wgrad_cluster() == 3 ? run_conv_wgrad_t<ConvWgradCfgC3>(G, X, dWt, B, M, C, P, st, what)
-                              : run_conv_wgrad_t<ConvWgradCfg>(G, X, dWt, B, M, C, P, st, what);
 }
 
 }  // namespace

@@ -9,7 +9,6 @@ rescales them on the device when the incoming grad is not 1
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import torch
 
@@ -260,7 +259,7 @@ def _scratch(device: torch.device, tag: str, nbytes: int) -> torch.Tensor:
 
 
 # --------------------------------------------------------------------------- hidden-state matching
-_LAYER_STREAMS = os.environ.get("DKD_LAYER_STREAMS", "1") != "0"
+_LAYER_STREAMS = True   # tests switch it off to get the single-stream reference
 _SIDE_STREAMS: dict = {}
 
 

@@ -20,8 +20,6 @@ import json
 import math
 import os
 import re
-import subprocess
-import sys
 import tempfile
 import zlib
 
@@ -33,8 +31,6 @@ from oracle.step import mixup_target
 from oracle.util import rel_err
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 LOSS_RTOL = 1e-5
 GRAD_RTOL = 1e-4
@@ -384,49 +380,6 @@ REACHABLE = (
 @pytest.mark.parametrize("case", ALL_CASES, ids=lambda c: c.id)
 def test_dispatch_case_matches_oracle(case):
     check_case(case)
-
-
-# --------------------------------------------------------------------------- ring fallback (DKD_LOGIT_RING=0)
-RING_OFF_SHAPES = [("bf16", 2048, 1000, "ring/8warp", 8), ("f32", 2048, 512, "ring/8warp", 4)]
-
-
-def _ring_off_cases(fam64: bool):
-    out = []
-    for dt, B, C, fam, vec in RING_OFF_SHAPES:
-        nv = -(-C // (64 * vec))
-        for labels, kd in MODES[:6]:
-            out.append(Case(dt, B, C, labels, kd, f"row64/nv{nv}" if fam64 else fam, vec))
-    return out
-
-
-def ring_off_child(out_path: str) -> None:
-    """Run in a process started with DKD_LOGIT_RING=0: the six modes at the ring shapes, results to out_path."""
-    res = {}
-    for case in _ring_off_cases(fam64=True):
-        got, kernels = profiled(lambda: run_op(case, *make_inputs(case)))
-        assert_launched(case, kernels)
-        res[case.id] = got
-    torch.save(res, out_path)
-
-
-def test_ring_disabled_runs_64_thread_modes():
-    """With the ring disabled (the variable is read once per process), B >= 1024 runs the six compiled modes of the
-    64-thread kernel.  They must match the oracle and the ring's losses in this process."""
-    with tempfile.TemporaryDirectory() as d:
-        out = os.path.join(d, "ring_off.pt")
-        code = ("import sys; sys.path.insert(0, sys.argv[1]); "
-                "from tests import test_logit_dispatch_matrix_gpu as m; m.ring_off_child(sys.argv[2])")
-        flags = ["-s"] if sys.flags.no_user_site else []
-        r = subprocess.run([sys.executable, *flags, "-c", code, ROOT, out], cwd=ROOT, capture_output=True, text=True,
-                           env={**os.environ, "DKD_LOGIT_RING": "0"}, timeout=600)
-        assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-        res = torch.load(out)
-    for c64, cring in zip(_ring_off_cases(fam64=True), _ring_off_cases(fam64=False)):
-        inputs = make_inputs(c64)
-        ref = oracle(c64, *(t.double() if t.is_floating_point() else t for t in inputs))
-        assert_matches(c64, res[c64.id], ref)
-        ring, _ = check_case(cring, inputs)
-        assert _close(res[c64.id][0], ring[0], LOSS_RTOL), (c64.id, res[c64.id][0], ring[0])
 
 
 # --------------------------------------------------------------------------- hard-KD ties placed per path
