@@ -1,5 +1,5 @@
 // Fused forward + dgrad of the hidden-state matching loss (CurKD early / mid, ViTKD mimicking; model/loss.py:376-393,
-// 277-289) for one Linear(192 -> 384) head:
+// 277-289) for one Linear(192 -> Dt) head, Dt = 384 (DeiT-Small teacher) or 768 (DeiT-Base teacher):
 //     Y = S W^T + b ;  d = Y - t ;  loss += sum d^2 ;  G = gscale * d (bf16 planes, kept for the weight-gradient GEMM) ;
 //     g_s = G W
 // in ONE persistent tcgen05 kernel per layer.
@@ -15,7 +15,8 @@
 //     (g_s += d_c W_c, K = the chunk's 64 teacher channels);
 //   * the residual chunk d_c goes TMEM -> registers (teacher subtracted, loss accumulated) -> a 128-byte-swizzled K-major
 //     shared-memory tile that is both the A operand of dgrad and the source of ONE tensor store per plane into the G planes
-//     (no per-thread global stores for G); the g_s accumulator (128 x 192 fp32) stays in TMEM across the six chunks.
+//     (no per-thread global stores for G); the g_s accumulator (128 x 192 fp32) stays in TMEM across the Dt / 64 chunks
+//     (6 at Dt = 384, 12 at Dt = 768).
 // Compared with the three-launch form (forward, dgrad, wgrad) the dgrad kernel's read of G (154 MB per layer in the fp32
 // mode) and one pass over the S planes are gone.
 //
@@ -24,6 +25,7 @@
 // its share of the S tile, and alternate 32-column pieces of g_s), warp 10 G tensor stores.
 // TMEM (512 columns): Y chunk double-buffered (2 x 64) | g_s (192) | S planes (2 x 96).
 // Shared memory: W ring 4 x 48 KB + d tile 32 KB = 224 KB (fp32 mode, P = 2 planes); 4 x 24 + 16 = 112 KB (bf16, P = 1).
+// Neither depends on the teacher width: a wider teacher only adds chunks to the walk over each row tile.
 #pragma once
 #include <stdlib.h>
 
@@ -31,12 +33,12 @@
 
 namespace dkd {
 
-template <int P_>
+template <int P_, int DT_>
 struct AlignFusedCfg {
   static constexpr int P = P_;                        // bf16 planes per operand (1: bf16, 2: bf16x3)
   static constexpr int TERMS = P_ == 2 ? 3 : 1;
-  static constexpr int DS = 192, DT = 384, CH = 64;   // student width, teacher width, teacher channels per chunk
-  static constexpr int NCH = DT / CH;                 // 6 chunks per tile
+  static constexpr int DS = 192, DT = DT_, CH = 64;   // student width, teacher width, teacher channels per chunk
+  static constexpr int NCH = DT / CH;                 // 6 (Dt = 384) or 12 (Dt = 768) chunks per tile
   static constexpr int KB = DS / 64;                  // 3 K blocks of the forward GEMM
   static constexpr int WST = 4;                       // W ring slots
   static constexpr int W_PLANE = KB * CH * 128;       // 24 KB: [KB][64 rows][128 B]
@@ -48,14 +50,16 @@ struct AlignFusedCfg {
   static constexpr uint32_t TM_Y = 0, TM_GS = 128, TM_S = 320;   // TMEM column offsets; S plane pl at TM_S + 96 * pl
   static constexpr int S_COLS = DS / 2;               // 96 packed columns per plane
   static_assert(SMEM <= 227 * 1024, "shared memory");
+  static_assert(DT % (2 * CH) == 0, "teacher width: whole pairs of 64-channel chunks");
+  static_assert(TM_GS == 2 * CH && TM_S == TM_GS + DS && TM_S + 2 * S_COLS == 512, "TMEM column map: Y (2 x 64) | g_s | S planes = 512");
 };
 
 struct AlignFusedParams {
-  CUtensorMap tmW;        // W planes [P][384][192], box {64, 64, 1}
-  CUtensorMap tmG;        // G planes [P][M][384], box {64, 128, 1} (stores)
+  CUtensorMap tmW;        // W planes [P][Dt][192], box {64, 64, 1}
+  CUtensorMap tmG;        // G planes [P][M][Dt], box {64, 128, 1} (stores)
   const __nv_bfloat16* S; // student planes [P][M][192]
-  const void* t;          // teacher [B, Tt, 384]
-  const float* bias;      // [384] or null
+  const void* t;          // teacher [B, Tt, Dt]
+  const float* bias;      // [Dt] or null
   void* g_s;              // [B, Ts, 192] dtype, or null
   double* partials;       // [gridDim.x]
   int64_t M;
@@ -330,7 +334,7 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) align_fused_kernel(const __gr
         chunk(c + 1, tb);
       }
       // the next tile's S planes go to tensor memory BEFORE this tile's g_s rows are read out: its forward MMAs then run
-      // under the g_s stores (the last forward of this tile retired before y_full of chunk 5, so s_empty has completed)
+      // under the g_s stores (the last forward of this tile retired before y_full of its last chunk, so s_empty has completed)
       if (tile_n < p.m_tiles) stage_S(tile_n, ti + 1);
       // ---- g_s rows of this tile: 6 pieces of 32 columns, alternating between the two groups
       mbar_wait(gs_full, ti & 1);
@@ -381,11 +385,11 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) align_fused_kernel(const __gr
 }
 
 // host: forward + dgrad of one layer.  `grid_out` = number of loss partials written.
-template <int P>
+template <int P, int DT>
 inline int align_fused_fwd_dgrad_t(const __nv_bfloat16* S, const __nv_bfloat16* Wp, const float* bias, const void* t, int t_is_bf16, int Tt,
                                    int t_off, int n_tok, __nv_bfloat16* G, double* partials, float gscale, void* g_s, int Ts, int s_off,
                                    int out_is_bf16, float gs_alpha, int64_t M, cudaStream_t st, int* grid_out, const char* what) {
-  using Cfg = AlignFusedCfg<P>;
+  using Cfg = AlignFusedCfg<P, DT>;
   AlignFusedParams p;
   int rc = make_plane_tmap(&p.tmW, Wp, P, Cfg::DT, Cfg::DS, Cfg::DS, (int64_t)Cfg::DT * Cfg::DS, Cfg::CH, what);
   if (rc != DKD_OK) return rc;
@@ -400,6 +404,18 @@ inline int align_fused_fwd_dgrad_t(const __nv_bfloat16* S, const __nv_bfloat16* 
   kern<<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(p);
   *grid_out = grid;
   return check_launch(what);
+}
+
+// host: the instantiation for (P, Dt); Dt in {384, 768} (the caller has checked it)
+inline int align_fused_fwd_dgrad(int P, int Dt, const __nv_bfloat16* S, const __nv_bfloat16* Wp, const float* bias, const void* t,
+                                 int t_is_bf16, int Tt, int t_off, int n_tok, __nv_bfloat16* G, double* partials, float gscale, void* g_s,
+                                 int Ts, int s_off, int out_is_bf16, float gs_alpha, int64_t M, cudaStream_t st, int* grid_out,
+                                 const char* what) {
+  auto run = [&](auto kern) {
+    return kern(S, Wp, bias, t, t_is_bf16, Tt, t_off, n_tok, G, partials, gscale, g_s, Ts, s_off, out_is_bf16, gs_alpha, M, st, grid_out, what);
+  };
+  if (Dt == 768) return P == 2 ? run(align_fused_fwd_dgrad_t<2, 768>) : run(align_fused_fwd_dgrad_t<1, 768>);
+  return P == 2 ? run(align_fused_fwd_dgrad_t<2, 384>) : run(align_fused_fwd_dgrad_t<1, 384>);
 }
 
 }  // namespace dkd

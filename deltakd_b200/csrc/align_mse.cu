@@ -1,7 +1,8 @@
 // Layer-wise hidden-state matching: loss += scale * || s[:,off:] W^T + b - t[:,off:] ||^2 with all gradients.
 // Reference: curkd_loss early / mid (model/loss.py:376-393) and the ViTKD mimicking term (loss.py:277-289)
-// — per layer `mse_loss(Linear(192->384)(student[:,1:]), teacher[:,2:], reduction='sum')` and its autograd
-// backward (grad of the student feature, of the Linear weight and of its bias).
+// — per layer `mse_loss(Linear(192->Dt)(student[:,1:]), teacher[:,2:], reduction='sum')` and its autograd
+// backward (grad of the student feature, of the Linear weight and of its bias).  Dt = 384 (DeiT-Small teacher) or
+// 768 (DeiT-Base teacher).
 //
 // Launch sequence per layer (all on `stream`, no host sync):
 //   1. tokens_to_planes   s[B,Ts,Ds] (patch tokens only) -> bf16 planes S[P][M][Ds]      (P = 1 bf16 | 2 bf16x3)
@@ -56,7 +57,9 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: precision %d", precision);
   DKD_REQUIRE(B > 0 && n_tok > 0 && s_off >= 0 && t_off >= 0 && Ts >= s_off + n_tok && Tt >= t_off + n_tok, DKD_E_SHAPE,
               "dkd_align_mse_fwdbwd: bad token geometry");
-  DKD_REQUIRE(Ds == 192 && Dt == 384, DKD_E_SHAPE, "dkd_align_mse_fwdbwd: built for DeiT-Tiny -> DeiT-Small widths (192 -> 384), got %d -> %d", Ds, Dt);
+  DKD_REQUIRE(Ds == 192 && (Dt == 384 || Dt == 768), DKD_E_SHAPE,
+              "dkd_align_mse_fwdbwd: built for widths 192 -> 384 (DeiT-Tiny -> DeiT-Small) and 192 -> 768 (DeiT-Tiny -> DeiT-Base), "
+              "got %d -> %d", Ds, Dt);
   DKD_REQUIRE(s && t && W && loss && workspace, DKD_E_SHAPE, "dkd_align_mse_fwdbwd: null pointer");
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "dkd_align_mse_fwdbwd: workspace must be 1024-byte aligned");
   DKD_REQUIRE((((uintptr_t)s | (uintptr_t)t | (uintptr_t)g_s) & 31) == 0, DKD_E_ALIGN, "%s: s, t and g_s must be 32-byte aligned (256-bit accesses)", "dkd_align_mse_fwdbwd");
@@ -76,10 +79,8 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   // 3. forward + residual + dgrad; the G planes it leaves feed step 5
   int grid = 0;
   const char* what = "dkd_align_mse_fwdbwd: fused forward + dgrad";
-  rc = P == 2 ? align_fused_fwd_dgrad_t<2>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
-                                           g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what)
-              : align_fused_fwd_dgrad_t<1>(ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale,
-                                           g_s, Ts, s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what);
+  rc = align_fused_fwd_dgrad(P, Dt, ws.S, ws.Wp, bias, t, dtype == DKD_BF16, Tt, t_off, n_tok, ws.G, ws.partials, 2.f * scale, g_s, Ts,
+                             s_off, dtype == DKD_BF16, 1.f, M, st, &grid, what);
   if (rc != DKD_OK) return rc;
   // 4. loss
   rc = launch_fold_partials(ws.partials, grid, scale, loss, st);

@@ -3,6 +3,7 @@
 //   align_forward_rows : A[M, Dt] fp32 = S W^T + bias                 (gemm_tn, StoreRows epilogue)
 //   align_dgrad        : g_s[:, off:, :] = alpha * G W                (gemm_tn, rows scattered, special tokens zeroed)
 //   align_wgrad        : g_W = alpha * G^T S, g_b = alpha * G^T 1     (gemm_nt split-K in 3-CTA clusters, ones-column trick)
+// Dt = 384 or 768 (the fused CurKD kernel of align_fused.cuh covers the forward and dgrad of align_mse).
 #pragma once
 #include "epilogues.cuh"
 #include "gemm_nt.cuh"
@@ -12,7 +13,8 @@ namespace dkd {
 
 using AlignCfg1 = GemmCfg<192, 1, 4, 2, 128, 1, 8>;   // one plane per stage (bf16 operands), 4-stage ring, 8 epilogue warps
 using AlignCfg2 = GemmCfg<192, 1, 2, 2, 128, 2, 8>;   // both planes per stage (bf16x3), 2 stages of 80 KB, 8 epilogue warps
-// wgrad: 3-CTA clusters (the three 128-wide teacher-channel tiles of one row split) with the S block multicast
+// wgrad: 3-CTA clusters (three 128-wide teacher-channel tiles of one row split) with the S block multicast; Dt = 768 has two
+// such tile groups per row split
 using AlignWgradCfg1 = GemmNtCfg<3, true, 208, 0, 4, 64, false, 1, 3>;
 // both planes per stage.  32 contraction rows per stage: 4 stages of 48 KB — with 64-row stages only two (96 KB each) fit and
 // every stage exposed a full TMA round trip (the kernel ran at 2.1 us per 64 rows against 0.65 us of MMA time)
@@ -73,10 +75,10 @@ inline int align_dgrad(const __nv_bfloat16* G, const __nv_bfloat16* Wt, void* g_
                 : align_dgrad_t<AlignCfg1>(G, Wt, g_s, M, n_tok, Ts, s_off, Ds, Dt, P, out_is_bf16, alpha, st, what);
 }
 
-template <class Cfg>
+template <class Cfg, int GROUPS>
 inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bfloat16* ones, float* g_W, float* g_b, int64_t M, int Ds, int Dt,
                          int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
-  using L = NtPlainLoader<Cfg>;
+  using L = NtPlainLoader<Cfg, GROUPS>;
   GemmNtParamsT<Cfg, L> p;
   int rc = make_plane_tmap(&p.ld.tmA, G, P, M, Dt, Dt, M * Dt, Cfg::KROWS, what);
   if (rc != DKD_OK) return rc;
@@ -98,15 +100,19 @@ inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bf
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
     return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
   }();
-  nt_make_splits(p.ld.total_row_blocks, resident, &p.ld.splits, &p.ld.row_blocks_per_split);
-  launch_gemm_nt<Cfg, L>(p, min(resident, p.ld.splits) * Cfg::CLUSTER, st);
+  // GROUPS work items (cluster tasks) per row split: about `resident` items in all, one wave of clusters
+  nt_make_splits(p.ld.total_row_blocks, resident / GROUPS, &p.ld.splits, &p.ld.row_blocks_per_split);
+  launch_gemm_nt<Cfg, L>(p, min(resident, GROUPS * p.ld.splits) * Cfg::CLUSTER, st);
   return check_launch(what);
 }
 
 inline int align_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bfloat16* ones, float* g_W, float* g_b, int64_t M, int Ds, int Dt,
                        int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
-  return P == 2 ? align_wgrad_t<AlignWgradCfg2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
-                : align_wgrad_t<AlignWgradCfg1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
+  if (Dt == 768)   // 6 teacher-channel tiles: two groups of 3
+    return P == 2 ? align_wgrad_t<AlignWgradCfg2, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
+                  : align_wgrad_t<AlignWgradCfg1, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
+  return P == 2 ? align_wgrad_t<AlignWgradCfg2, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
+                : align_wgrad_t<AlignWgradCfg1, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
 }
 
 }  // namespace dkd

@@ -299,16 +299,18 @@ struct NtItem {
 };
 
 // Plain loader: A = planes [P][R][NA_total], B = planes [P][R][NB_total], 3-D maps {cols, rows, planes}, box {64, KROWS, 1}.
+// GROUPS_ (cluster form only): the A column tiles are GROUPS_ groups of CLUSTER tiles (na_tiles == GROUPS_ * CLUSTER).
 struct NtPlainParams {
   CUtensorMap tmA, tmB, tmOnes;
   int na_tiles, splits, row_blocks_per_split, total_row_blocks, b_col0, ldd;
 };
-template <class Cfg>
+template <class Cfg, int GROUPS_ = 1>
 struct NtPlainLoader {
   using Params = NtPlainParams;
   using Item = NtItem;
   static constexpr uint32_t TX_BYTES = Cfg::STAGE_BYTES;
-  static __device__ __forceinline__ int num_items(const Params& p) { return Cfg::CLUSTER > 1 ? p.splits : p.na_tiles * p.splits; }
+  static_assert(GROUPS_ >= 1 && (GROUPS_ == 1 || Cfg::CLUSTER > 1), "tile groups are a cluster-form schedule");
+  static __device__ __forceinline__ int num_items(const Params& p) { return Cfg::CLUSTER > 1 ? GROUPS_ * p.splits : p.na_tiles * p.splits; }
   static __device__ __forceinline__ void prefetch(const Params& p) {
     sm100::tma_prefetch_desc(&p.tmA);
     sm100::tma_prefetch_desc(&p.tmB);
@@ -340,16 +342,20 @@ struct NtPlainLoader {
     if constexpr (Cfg::ONES)  // plane 0 of the ones tile is {1,0,0,...}; its lo plane is all zero
       sm100::tma_load_3d(b + (size_t)Cfg::NB_BOXES * Cfg::BOX_BYTES, &p.tmOnes, bar, 0, 0, pb);
   }
-  // ---- cluster form: the CLUSTER CTAs of a cluster are the A column tiles (na_tiles == CLUSTER) of ONE row split: they
-  // contract over the same rows of B, so CTA `crank` fetches B box `crank` and multicasts it (NB_BOXES == CLUSTER).
-  static __device__ __forceinline__ int num_items_cluster(const Params& p) { return p.splits; }
+  // ---- cluster form: a work item is one (tile group, row split) pair, and the CLUSTER CTAs of a cluster are the A column
+  // tiles of ONE group (CTA `crank` of group g owns tile g * CLUSTER + crank) over ONE row split: they contract over the
+  // same rows of B, so CTA `crank` fetches B box `crank` and multicasts it (NB_BOXES == CLUSTER).  GROUPS_ = 1: the
+  // cluster covers all A tiles (na_tiles == CLUSTER) and an item is a row split.
+  static __device__ __forceinline__ int num_items_cluster(const Params& p) { return GROUPS_ * p.splits; }
   static __device__ __forceinline__ void decode_cluster(const Params& p, int item, int crank, Item& it) {
-    it.rb0 = item * p.row_blocks_per_split;
+    const int group = item % GROUPS_, split = item / GROUPS_;
+    const int tile = group * Cfg::CLUSTER + crank;
+    it.rb0 = split * p.row_blocks_per_split;
     it.rb1 = min(it.rb0 + p.row_blocks_per_split, p.total_row_blocks);
-    it.a_col0 = crank * 128;
+    it.a_col0 = tile * 128;
     it.b_col0 = p.b_col0;
-    it.d_off = (int64_t)crank * 128 * p.ldd;
-    it.dcol_off = crank * 128;
+    it.d_off = (int64_t)tile * 128 * p.ldd;
+    it.dcol_off = tile * 128;
     it.aux = 0;
   }
   static __device__ __forceinline__ void issue_planes_cluster(const Params& p, const Item& it, int pa, int pb, int rb, uint8_t* a, uint8_t* b,

@@ -273,7 +273,8 @@ int dkd_wass_l1_fwdbwd(const void* s, const void* t, const float* W, const float
   DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
   DKD_REQUIRE(B > 0 && n_tok > 0 && n_tok <= kMaxTok && s_off >= 0 && t_off >= 0 && Ts >= s_off + n_tok && Tt >= t_off + n_tok,
               DKD_E_SHAPE, "%s: bad token geometry (n_tok <= %d)", fn, kMaxTok);
-  DKD_REQUIRE(Ds == 192 && Dt == 384, DKD_E_SHAPE, "%s: built for widths 192 -> 384, got %d -> %d", fn, Ds, Dt);
+  DKD_REQUIRE(Ds == 192 && (Dt == 384 || Dt == 768), DKD_E_SHAPE,
+              "%s: built for widths 192 -> 384 (DeiT-Tiny -> DeiT-Small) and 192 -> 768 (DeiT-Tiny -> DeiT-Base), got %d -> %d", fn, Ds, Dt);
   DKD_REQUIRE(s && t && W && loss && workspace, DKD_E_SHAPE, "%s: null pointer", fn);
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "%s: workspace must be 1024-byte aligned", fn);
   DKD_REQUIRE((((uintptr_t)s | (uintptr_t)t | (uintptr_t)g_s) & 31) == 0, DKD_E_ALIGN, "%s: s, t and g_s must be 32-byte aligned (256-bit accesses)", "dkd_wass_l1_fwdbwd");

@@ -3,8 +3,9 @@
 The reference builds its student and teacher with `timm.create_model` (model/models.py:59-75); timm is not in this
 image and the models are outside the hot path (SURVEY.md §8: plain PyTorch is fine; `row_ops="dkd"` swaps the
 HBM-bound LayerNorm / bias-gradient / head-relayout passes for libdeltakd_sm100 kernels, §8f rank 1).  This file
-provides random-init stand-ins of `deit_tiny[_distilled]_patch16_224` (192-d, 3 heads) and
-`deit_small_distilled_patch16_224` (384-d, 6 heads) exposing exactly what the loss path touches:
+provides random-init stand-ins of `deit_tiny[_distilled]_patch16_224` (192-d, 3 heads),
+`deit_small[_distilled]_patch16_224` (384-d, 6 heads) and `deit_base[_distilled]_patch16_224` (768-d, 12 heads; the
+wider teacher of the 192 -> 768 feature losses) exposing exactly what the loss path touches:
 `.embed_dim`, `.blocks[i].mlp` (hooked by forward_with_features, models.py:185-193), `.head` / `.head_dist`,
 `set_distilled_training` (models.py:97), and timm's output convention (distilled + training + distilled_training
 -> (cls_logits, dist_logits); otherwise their mean / the single head).
@@ -139,12 +140,14 @@ _ZOO = {
     "deit_tiny_distilled_patch16_224": dict(embed_dim=192, depth=12, num_heads=3, distilled=True),
     "deit_small_patch16_224": dict(embed_dim=384, depth=12, num_heads=6, distilled=False),
     "deit_small_distilled_patch16_224": dict(embed_dim=384, depth=12, num_heads=6, distilled=True),
+    "deit_base_patch16_224": dict(embed_dim=768, depth=12, num_heads=12, distilled=False),
+    "deit_base_distilled_patch16_224": dict(embed_dim=768, depth=12, num_heads=12, distilled=True),
 }
 
 
 def create_model(name: str, num_classes: int = 1000, row_ops: str = "aten", **_) -> DeiT:
     """Stand-in for timm.create_model(name, pretrained=False, num_classes=...) restricted to the DeiT variants the
-    reference's exp/*.sh scripts use.  `row_ops="dkd"` builds the same model (same state_dict) on libdeltakd_sm100's
+    reference's exp/*.sh scripts use, plus the DeiT-Base teacher.  `row_ops="dkd"` builds the same model (same state_dict) on libdeltakd_sm100's
     LayerNorm / bias-gradient / head-relayout kernels — CUDA only."""
     if name not in _ZOO:
         raise ValueError(f"unknown model {name}; available: {sorted(_ZOO)}")

@@ -336,23 +336,36 @@ class _AlignMseLayers(torch.autograd.Function):
         return (None, None, None, None, None, *gs, *([None] * n), *gw, *gb)
 
 
-SUPPORTED_WIDTHS = (192, 384)     # student -> teacher embedding widths the tcgen05 tile configurations are built for
+# (student, teacher) embedding widths each feature entry point's tcgen05 tile configurations are built for
+_DEIT_TS = (192, 384)   # deit_tiny -> deit_small, the pair of every exp/*.sh script
+_DEIT_TB = (192, 768)   # deit_tiny -> deit_base
+_PAIR_NAMES = {_DEIT_TS: "deit_tiny -> deit_small", _DEIT_TB: "deit_tiny -> deit_base"}
+SUPPORTED_PAIRS = {
+    "dkd_align_mse": (_DEIT_TS, _DEIT_TB),
+    "dkd_wass_l1": (_DEIT_TS, _DEIT_TB),
+    "dkd_align_nmse": (_DEIT_TS,),
+    "dkd_wass_sinkhorn": (_DEIT_TS,),
+    "masked generation": (_DEIT_TS,),
+    "LRKD": (_DEIT_TS,),
+}
 SUPPORTED_GRID_TOKENS = 196       # 14 x 14 patch grid (224-px inputs, patch 16) for the generator conv / Sinkhorn kernels
 
 
-def _check_feature_pair(s, t, s_off, t_off, op: str = "feature loss", grid_tokens: bool = False):
-    """Validates one (student, teacher) feature pair and states the supported model matrix in the error: the feature
-    kernels are compiled for DeiT-Tiny -> DeiT-Small widths (192 -> 384), which is what all 19 exp/*.sh scripts of the
-    reference use; other timm pairs (e.g. a 768-wide teacher, 384-px inputs) are rejected here, at the first call,
-    instead of failing deep inside a launch."""
+def _check_feature_pair(s, t, s_off, t_off, op: str, grid_tokens: bool = False):
+    """Validates one (student, teacher) feature pair for the entry point `op` (a key of SUPPORTED_PAIRS) and states the
+    pairs it supports in the error: every feature loss is built for DeiT-Tiny -> DeiT-Small widths (192 -> 384), which
+    is what all 19 exp/*.sh scripts of the reference use, and the hidden-state matching and WassKD-l1 losses also for a
+    DeiT-Base teacher (192 -> 768); other timm pairs (e.g. a 384-wide student, 384-px inputs) are rejected here, at the
+    first call, instead of failing deep inside a launch."""
     _require_cuda(s, t)
     if s.dim() != 3 or t.dim() != 3 or s.shape[0] != t.shape[0]:
         raise ValueError(f"features must be [B, tokens, dim]; got {tuple(s.shape)} and {tuple(t.shape)}")
     if s.shape[1] - s_off != t.shape[1] - t_off:
         raise ValueError(f"patch-token counts differ: student {s.shape[1] - s_off} vs teacher {t.shape[1] - t_off}")
-    if (s.shape[2], t.shape[2]) != SUPPORTED_WIDTHS:
-        raise ValueError(f"deltakd_b200 {op}: built for student/teacher widths {SUPPORTED_WIDTHS[0]} -> {SUPPORTED_WIDTHS[1]} "
-                         f"(deit_tiny -> deit_small, the pair of every exp/*.sh script); got {s.shape[2]} -> {t.shape[2]}. "
+    pairs = SUPPORTED_PAIRS[op]
+    if (s.shape[2], t.shape[2]) not in pairs:
+        built = " and ".join(f"{ds} -> {dt} ({_PAIR_NAMES[(ds, dt)]})" for ds, dt in pairs)
+        raise ValueError(f"deltakd_b200 {op}: built for student/teacher widths {built}; got {s.shape[2]} -> {t.shape[2]}. "
                          "See INTEGRATION.md 'Supported model matrix'.")
     if grid_tokens and s.shape[1] - s_off != SUPPORTED_GRID_TOKENS:
         raise ValueError(f"deltakd_b200 {op}: built for {SUPPORTED_GRID_TOKENS} patch tokens (14 x 14 grid: 224-px inputs, patch 16); "

@@ -124,7 +124,8 @@ DKD_API int dkd_scale_if_not_one(void* x, int64_t n, void* x2, int64_t n2, int d
  *   W [Dt,Ds], bias [Dt], g_W, g_b, loss : fp32 ;  g_s : `dtype`  (any g_* may be NULL)
  *   precision : DKD_PREC_BF16 | DKD_PREC_BF16X3 (tcgen05 bf16 passes, fp32 accumulate in TMEM)
  *   workspace : >= dkd_align_mse_workspace_bytes(...) bytes, 1024-byte aligned, contents don't matter
- * Built for the DeiT-Tiny -> DeiT-Small widths: Ds = 192, Dt = 384.
+ * Built for Ds = 192 with Dt = 384 (DeiT-Tiny -> DeiT-Small) or Dt = 768 (DeiT-Tiny -> DeiT-Base); any other pair
+ * returns DKD_E_SHAPE.
  */
 DKD_API size_t dkd_align_mse_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision);
 DKD_API int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const float* bias, int64_t B, int Ts,
@@ -139,7 +140,7 @@ DKD_API int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, c
  * Replaces, per layer of the diffkd branch (model/loss.py:112-116, 139-140, 149), the alignment Linear, the two
  * per-token L2 normalisations and `F.mse_loss(s_feat, t_feat)` with their backward; the caller folds 1/numel into
  * `scale` and applies the data-dependent weight w_t.mean() (a device scalar) through the autograd rescale.
- * Same argument conventions as dkd_align_mse_fwdbwd.  The noise-prediction term of that branch
+ * Same argument conventions as dkd_align_mse_fwdbwd, but built for Ds = 192, Dt = 384 only.  The noise-prediction term of that branch
  * (`student.denoise_fn`, an nn.Module with Dropout) stays a module call.
  */
 DKD_API size_t dkd_align_nmse_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision);
@@ -156,6 +157,8 @@ DKD_API int dkd_align_nmse_fwdbwd(const void* s, const void* t, const float* W, 
  * Replaces model/loss.py:187-199 (torch.sort over dim=1 of both tensors, mean |diff|) and its backward;
  * the caller folds 5/(3*B*n_tok*Dt) into `scale`.  Same argument conventions as dkd_align_mse_fwdbwd;
  * n_tok <= 256.  Ties in the student sort are ordered by token index.
+ * Built for Ds = 192 with Dt = 384 (DeiT-Tiny -> DeiT-Small) or Dt = 768 (DeiT-Tiny -> DeiT-Base); any other pair
+ * returns DKD_E_SHAPE.
  */
 DKD_API size_t dkd_wass_l1_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision);
 DKD_API int dkd_wass_l1_fwdbwd(const void* s, const void* t, const float* W, const float* bias, int64_t B, int Ts, int s_off,
