@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libdeltakd_sm100.so")
 
 F32, BF16 = 0, 1
 PREC_BF16, PREC_BF16X3 = 0, 1
+PREC_DETERMINISTIC = 0x100   # OR'ed into the precision of the gradient-bearing feature entry points
 OK = 0
 
 if not os.path.exists(LIB_PATH):

@@ -23,9 +23,10 @@ size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 struct Workspace {
   __nv_bfloat16 *S, *Wp, *G, *ones;
   double* partials;
+  float* wpart;   // deterministic mode: per-split weight-gradient slots (align_wgrad), appended last
   size_t bytes;
 };
-Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
+Workspace carve(void* base, int64_t M, int Ds, int Dt, int P, bool det) {
   Workspace w;
   size_t off = 0;
   auto take = [&](size_t n) { size_t o = off; off = align_up(off + n, 1024); return reinterpret_cast<char*>(base) + o; };
@@ -34,6 +35,7 @@ Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
   w.Wp = reinterpret_cast<__nv_bfloat16*>(take((size_t)P * Dt * Ds * 2));
   w.ones = reinterpret_cast<__nv_bfloat16*>(take((size_t)2 * 64 * 64 * 2));
   w.partials = reinterpret_cast<double*>(take((size_t)kNumSMs * sizeof(double)));
+  w.wpart = det ? reinterpret_cast<float*>(take(align_wgrad_part_bytes(M, Ds, Dt, P))) : nullptr;
   w.bytes = off;
   return w;
 }
@@ -44,7 +46,7 @@ Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
 extern "C" {
 
 size_t dkd_align_mse_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision) {
-  return dkd::carve(nullptr, B * n_tok, Ds, Dt, precision == DKD_PREC_BF16X3 ? 2 : 1).bytes;
+  return dkd::carve(nullptr, B * n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision)).bytes;
 }
 
 int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const float* bias, int64_t B, int Ts, int s_off,
@@ -54,7 +56,7 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   int rc = dkd_check_device();
   if (rc != DKD_OK) return rc;
   DKD_REQUIRE(dtype == DKD_F32 || dtype == DKD_BF16, DKD_E_DTYPE, "dkd_align_mse_fwdbwd: dtype %d", dtype);
-  DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: precision %d", precision);
+  DKD_REQUIRE(prec_valid(precision), DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: precision %d", precision);
   DKD_REQUIRE(B > 0 && n_tok > 0 && s_off >= 0 && t_off >= 0 && Ts >= s_off + n_tok && Tt >= t_off + n_tok, DKD_E_SHAPE,
               "dkd_align_mse_fwdbwd: bad token geometry");
   DKD_REQUIRE(Ds == 192 && (Dt == 384 || Dt == 768), DKD_E_SHAPE,
@@ -63,10 +65,10 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   DKD_REQUIRE(s && t && W && loss && workspace, DKD_E_SHAPE, "dkd_align_mse_fwdbwd: null pointer");
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "dkd_align_mse_fwdbwd: workspace must be 1024-byte aligned");
   DKD_REQUIRE((((uintptr_t)s | (uintptr_t)t | (uintptr_t)g_s) & 31) == 0, DKD_E_ALIGN, "%s: s, t and g_s must be 32-byte aligned (256-bit accesses)", "dkd_align_mse_fwdbwd");
-  const int P = precision == DKD_PREC_BF16X3 ? 2 : 1;
+  const int P = prec_planes(precision);
   const int64_t M = B * n_tok;
   DKD_REQUIRE(M < (1ll << 31) - 256, DKD_E_SHAPE, "dkd_align_mse_fwdbwd: too many rows");
-  Workspace ws = carve(workspace, M, Ds, Dt, P);
+  Workspace ws = carve(workspace, M, Ds, Dt, P, prec_deterministic(precision));
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "dkd_align_mse_fwdbwd: workspace %zu < %zu", workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
 
@@ -88,7 +90,7 @@ int dkd_align_mse_fwdbwd(const void* s, const void* t, const float* W, const flo
   // 5. g_W = G^T S, g_b = G^T 1
   if (g_W || g_b) {
     DKD_REQUIRE(g_W != nullptr, DKD_E_UNSUPPORTED, "dkd_align_mse_fwdbwd: g_b without g_W is not supported");
-    rc = align_wgrad(ws.G, ws.S, ws.ones, g_W, g_b, M, Ds, Dt, P, 1.f, st, "dkd_align_mse_fwdbwd: wgrad GEMM");
+    rc = align_wgrad(ws.G, ws.S, ws.ones, g_W, g_b, M, Ds, Dt, P, 1.f, st, "dkd_align_mse_fwdbwd: wgrad GEMM", 0, ws.wpart);
     if (rc != DKD_OK) return rc;
   }
   return DKD_OK;

@@ -2,7 +2,8 @@
 // activations themselves (WassKD): forward rows, and the backward from a gradient-plane tensor G[P][M][Dt].
 //   align_forward_rows : A[M, Dt] fp32 = S W^T + bias                 (gemm_tn, StoreRows epilogue)
 //   align_dgrad        : g_s[:, off:, :] = alpha * G W                (gemm_tn, rows scattered, special tokens zeroed)
-//   align_wgrad        : g_W = alpha * G^T S, g_b = alpha * G^T 1     (gemm_nt split-K in 3-CTA clusters, ones-column trick)
+//   align_wgrad        : g_W = alpha * G^T S, g_b = alpha * G^T 1     (gemm_nt split-K in 3-CTA clusters, ones-column trick;
+//                        float atomics, or per-split slots and a fixed-order fold in deterministic mode)
 // Dt = 384 or 768 (the fused CurKD kernel of align_fused.cuh covers the forward and dgrad of align_mse).
 #pragma once
 #include "epilogues.cuh"
@@ -75,9 +76,31 @@ inline int align_dgrad(const __nv_bfloat16* G, const __nv_bfloat16* Wt, void* g_
                 : align_dgrad_t<AlignCfg1>(G, Wt, g_s, M, n_tok, Ts, s_off, Ds, Dt, P, out_is_bf16, alpha, st, what);
 }
 
+// Deterministic mode (`part` non-null): the split count depends on the shapes only (kNumSMs / CLUSTER clusters instead of
+// the device's resident-cluster count), every work item stores its tile and its ones column with plain stores
+// into slot part[split][nt_slot_floats(Dt * Ds + Dt)], and fold_splits_kernel adds the slots in split order in fp64 and applies alpha.
+template <class Cfg, int GROUPS>
+inline void align_wgrad_splits(int64_t M, int want, int* splits, int* per_split) {
+  nt_make_splits((int)((M + Cfg::KROWS - 1) / Cfg::KROWS), want / GROUPS, splits, per_split);
+}
+
+template <class Cfg, int GROUPS>
+inline size_t align_wgrad_part_bytes_t(int64_t M, int Ds, int Dt) {
+  int splits, per;
+  align_wgrad_splits<Cfg, GROUPS>(M, kNumSMs / Cfg::CLUSTER, &splits, &per);
+  return (size_t)splits * nt_slot_floats((int64_t)Dt * Ds + Dt) * sizeof(float);
+}
+
+// bytes of the deterministic-mode partial slots of align_wgrad
+inline size_t align_wgrad_part_bytes(int64_t M, int Ds, int Dt, int P) {
+  if (Dt == 768)
+    return P == 2 ? align_wgrad_part_bytes_t<AlignWgradCfg2, 2>(M, Ds, Dt) : align_wgrad_part_bytes_t<AlignWgradCfg1, 2>(M, Ds, Dt);
+  return P == 2 ? align_wgrad_part_bytes_t<AlignWgradCfg2, 1>(M, Ds, Dt) : align_wgrad_part_bytes_t<AlignWgradCfg1, 1>(M, Ds, Dt);
+}
+
 template <class Cfg, int GROUPS>
 inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bfloat16* ones, float* g_W, float* g_b, int64_t M, int Ds, int Dt,
-                         int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
+                         int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero, float* part) {
   using L = NtPlainLoader<Cfg, GROUPS>;
   GemmNtParamsT<Cfg, L> p;
   int rc = make_plane_tmap(&p.ld.tmA, G, P, M, Dt, Dt, M * Dt, Cfg::KROWS, what);
@@ -88,9 +111,15 @@ inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bf
   if (rc != DKD_OK) return rc;
   rc = launch_fill_ones_tile(ones, st);
   if (rc != DKD_OK) return rc;
-  cudaMemsetAsync(g_W, 0, (size_t)Dt * Ds * sizeof(float), st);
-  if (g_b) cudaMemsetAsync(g_b, 0, (size_t)Dt * sizeof(float), st);
-  p.ep.D = g_W; p.ep.Dcol = g_b; p.ep.ldd = Ds; p.ep.alpha = alpha;
+  const int64_t slot = nt_slot_floats((int64_t)Dt * Ds + Dt);
+  if (part) {
+    p.ep.D = part; p.ep.Dcol = g_b ? part + (int64_t)Dt * Ds : nullptr; p.ep.alpha = 1.f; p.ep.store = 1; p.ep.split_stride = slot;
+  } else {
+    cudaMemsetAsync(g_W, 0, (size_t)Dt * Ds * sizeof(float), st);
+    if (g_b) cudaMemsetAsync(g_b, 0, (size_t)Dt * sizeof(float), st);
+    p.ep.D = g_W; p.ep.Dcol = g_b; p.ep.alpha = alpha;
+  }
+  p.ep.ldd = Ds;
   p.ld.ldd = Ds; p.ld.na_tiles = Dt / 128; p.ld.b_col0 = 0;
   p.ld.total_row_blocks = (int)((M + Cfg::KROWS - 1) / Cfg::KROWS);
   p.nterms = P == 2 ? 3 : 1;
@@ -100,19 +129,24 @@ inline int align_wgrad_t(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bf
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
     return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
   }();
-  // GROUPS work items (cluster tasks) per row split: about `resident` items in all, one wave of clusters
-  nt_make_splits(p.ld.total_row_blocks, resident / GROUPS, &p.ld.splits, &p.ld.row_blocks_per_split);
+  // GROUPS work items (cluster tasks) per row split: about `resident` items in all, one wave of clusters.  The deterministic
+  // split count is fixed by the shapes; its grid stays at the resident count, since each item owns its slot and which
+  // cluster computes it cannot change a bit
+  align_wgrad_splits<Cfg, GROUPS>(M, part ? kNumSMs / Cfg::CLUSTER : resident, &p.ld.splits, &p.ld.row_blocks_per_split);
   launch_gemm_nt<Cfg, L>(p, min(resident, GROUPS * p.ld.splits) * Cfg::CLUSTER, st);
-  return check_launch(what);
+  rc = check_launch(what);
+  if (rc != DKD_OK || !part) return rc;
+  return launch_fold_splits(part, p.ld.splits, slot, (int64_t)Dt * Ds, g_W, g_b ? Dt : 0, g_b, alpha, st);
 }
 
+// part: null = split-K reduction with float atomics into g_W / g_b; else deterministic mode, align_wgrad_part_bytes(...) bytes
 inline int align_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* S, __nv_bfloat16* ones, float* g_W, float* g_b, int64_t M, int Ds, int Dt,
-                       int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0) {
+                       int P, float alpha, cudaStream_t st, const char* what, int g_lo_zero = 0, float* part = nullptr) {
   if (Dt == 768)   // 6 teacher-channel tiles: two groups of 3
-    return P == 2 ? align_wgrad_t<AlignWgradCfg2, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
-                  : align_wgrad_t<AlignWgradCfg1, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
-  return P == 2 ? align_wgrad_t<AlignWgradCfg2, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero)
-                : align_wgrad_t<AlignWgradCfg1, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what);
+    return P == 2 ? align_wgrad_t<AlignWgradCfg2, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero, part)
+                  : align_wgrad_t<AlignWgradCfg1, 2>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, 0, part);
+  return P == 2 ? align_wgrad_t<AlignWgradCfg2, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, g_lo_zero, part)
+                : align_wgrad_t<AlignWgradCfg1, 1>(G, S, ones, g_W, g_b, M, Ds, Dt, P, alpha, st, what, 0, part);
 }
 
 }  // namespace dkd

@@ -27,6 +27,15 @@ int check_launch(const char* what);  // cudaGetLastError -> DKD_E_LAUNCH
 
 constexpr int kNumSMs = 148;  // B200
 
+// `precision` of the gradient-bearing feature entry points: DKD_PREC_BF16 | DKD_PREC_BF16X3, optionally
+// | DKD_PREC_DETERMINISTIC; any other bit is unsupported
+inline bool prec_valid(int precision) {
+  const int base = precision & ~DKD_PREC_DETERMINISTIC;
+  return base == DKD_PREC_BF16 || base == DKD_PREC_BF16X3;
+}
+inline int prec_planes(int precision) { return (precision & ~DKD_PREC_DETERMINISTIC) == DKD_PREC_BF16X3 ? 2 : 1; }
+inline bool prec_deterministic(int precision) { return (precision & DKD_PREC_DETERMINISTIC) != 0; }
+
 // ---- programmatic dependent launch ---------------------------------------------
 // A kernel launched by launch_pdl may start while its predecessor on the stream is still running (its CTAs are resident
 // and have called grid_dep_launch, or have exited), so launch latency and prologue overlap the predecessor's tail.  It

@@ -164,6 +164,7 @@ struct NtConvLoader {
   static __device__ __forceinline__ void decode_cluster(const Params& p, int item, int crank, Item& it) {
     const int combo = item % COMBOS_CLUSTER, split = item / COMBOS_CLUSTER;
     const int tap = combo >> 1, ci_half = combo & 1;
+    it.split = split;
     it.rb0 = split * p.row_blocks_per_split;
     it.rb1 = min(it.rb0 + p.row_blocks_per_split, p.total_row_blocks);
     it.a_col0 = crank * 128;

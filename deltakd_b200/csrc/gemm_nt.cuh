@@ -5,7 +5,9 @@
 //
 // Work item = (output tile, row split); the Loader policy decodes it.  Each CTA loops over its items;
 // per item it accumulates over the split's row blocks in TMEM (one 128 x NB fp32 tile) and the epilogue
-// adds the tile into fp32 D with red.global.add (D is zeroed by the host wrapper).  Warp roles as in
+// adds the tile into fp32 D with red.global.add (D is zeroed by the host wrapper), or, with `store` and `split_stride`,
+// writes it with plain stores into the split's own slot of a partial buffer that fold_splits_kernel then reduces in split
+// order (the deterministic mode: no float add depends on CTA timing).  Warp roles as in
 // gemm_tn.cuh: warp 0 TMA producer, warp 1 MMA issuer, warps 2-5 epilogue.
 //
 // The B operand may carry one extra box from a constant "ones" tile (column 0 = 1): its first 16
@@ -50,10 +52,11 @@ struct GemmNtCfg {
 
 struct NtEpilogueParams {
   float* D = nullptr;     // fp32, += via red.add (or plain stores when `store`)
-  float* Dcol = nullptr;  // += column NB_DATA of the tile (ones trick), or null
+  float* Dcol = nullptr;  // += column NB_DATA of the tile (ones trick), or null; plain stores when `store`
   int ldd = 0;
   float alpha = 1.f;
   int store = 0;          // 1: the tile is written with plain stores (each item owns its output, e.g. per-split partials)
+  int64_t split_stride = 0;  // elements between the per-split slots of D and Dcol (items carry their split index)
   int rows_valid = 128;   // output rows of the 128-row tile that exist (A narrower than 128 columns)
   __nv_bfloat16* Dplanes = nullptr;  // if set: the tile is written as bf16 hi(/lo) planes here instead of fp32 D
   int64_t plane_stride = 0;
@@ -201,7 +204,8 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) gemm_nt_kernel(const __grid_c
       mbar_wait(acc_full, aph);
       tc_fence_after();
       const uint32_t t_acc = tmem_base + ((uint32_t)(quad * 32) << 16);
-      float* drow = p.ep.D + it.d_off + (size_t)row * p.ep.ldd;
+      const int64_t slot = (int64_t)it.split * p.ep.split_stride;
+      float* drow = p.ep.D + slot + it.d_off + (size_t)row * p.ep.ldd;
       const bool row_ok = row < p.ep.rows_valid && row < it.rows;
 #pragma unroll 1
       for (int c0 = 0; c0 < Cfg::NB_DATA; c0 += 32) {
@@ -230,7 +234,10 @@ __global__ void __launch_bounds__(Cfg::THREADS, 1) gemm_nt_kernel(const __grid_c
         float v[32];
         tmem_ld32(t_acc + Cfg::NB_DATA - 16, v);  // columns NB_DATA-16 .. NB_DATA+15 (inside the allocation)
         tmem_ld_wait();
-        if (row_ok && p.ep.Dcol && it.dcol_off >= 0) atomicAdd(p.ep.Dcol + it.dcol_off + row, v[16] * p.ep.alpha);
+        if (row_ok && p.ep.Dcol && it.dcol_off >= 0) {
+          if (p.ep.store) p.ep.Dcol[slot + it.dcol_off + row] = v[16] * p.ep.alpha;
+          else atomicAdd(p.ep.Dcol + it.dcol_off + row, v[16] * p.ep.alpha);
+        }
       }
       tc_fence_before();
       __syncwarp();
@@ -296,6 +303,7 @@ struct NtItem {
   int dcol_off;      // offset into Dcol, or -1
   int aux;           // loader specific (e.g. filter tap)
   int rows = 128;    // output rows of this item's tile that exist (<= 128)
+  int split = 0;     // row split: selects the partial slot (NtEpilogueParams::split_stride)
 };
 
 // Plain loader: A = planes [P][R][NA_total], B = planes [P][R][NB_total], 3-D maps {cols, rows, planes}, box {64, KROWS, 1}.
@@ -317,6 +325,7 @@ struct NtPlainLoader {
   }
   static __device__ __forceinline__ void decode(const Params& p, int item, Item& it) {
     const int tile = item % p.na_tiles, split = item / p.na_tiles;
+    it.split = split;
     it.rb0 = split * p.row_blocks_per_split;
     it.rb1 = min(it.rb0 + p.row_blocks_per_split, p.total_row_blocks);
     it.a_col0 = tile * 128;
@@ -350,6 +359,7 @@ struct NtPlainLoader {
   static __device__ __forceinline__ void decode_cluster(const Params& p, int item, int crank, Item& it) {
     const int group = item % GROUPS_, split = item / GROUPS_;
     const int tile = group * Cfg::CLUSTER + crank;
+    it.split = split;
     it.rb0 = split * p.row_blocks_per_split;
     it.rb1 = min(it.rb0 + p.row_blocks_per_split, p.total_row_blocks);
     it.a_col0 = tile * 128;
@@ -376,6 +386,11 @@ struct NtPlainLoader {
     issue_planes_cluster(p, it, pa, pb, rb, a, b, bar, crank);
   }
 };
+
+// host: elements between the per-split slots of a deterministic-mode partial buffer that holds `n` floats per split.
+// The store epilogue writes the tile with 16-byte vector stores from the slot base, so a slot starts on a 128-byte
+// boundary (whole L2 sectors) whatever `n` is (e.g. LRKD's rank * (Ds + 1) for an odd rank).
+inline int64_t nt_slot_floats(int64_t n) { return (n + 31) / 32 * 32; }
 
 // host: split `total_row_blocks` over about `want` splits with no empty split
 inline void nt_make_splits(int total_row_blocks, int want, int* splits, int* per_split) {

@@ -791,11 +791,19 @@ struct Workspace {
   double *gsum, *W, *sumsq, *partials;
   unsigned* bar;
   unsigned long long* offmax;
+  float* wpart;   // deterministic mode only: per-split slots of the head wgrad [split][nt_slot_floats(rank * (Ds + 1))], appended last
   size_t bytes;
 };
 constexpr int kSumsqBlocks = 296;
 
-Workspace carve(void* base, int L, int64_t M, int Ds, int BN, int PT, int P) {
+// head wgrad row splits: one per SM (a function of M alone)
+int wgrad_splits(int64_t M, int* per_split) {
+  int splits;
+  nt_make_splits((int)((M + WgradCfg::KROWS - 1) / WgradCfg::KROWS), kNumSMs, &splits, per_split);
+  return splits;
+}
+
+Workspace carve(void* base, int L, int64_t M, int Ds, int BN, int PT, int P, bool det) {
   Workspace w;
   size_t off = 0;
   auto take = [&](size_t n) { size_t o = off; off = align_up(off + n, 1024); return reinterpret_cast<char*>(base) + o; };
@@ -813,6 +821,8 @@ Workspace carve(void* base, int L, int64_t M, int Ds, int BN, int PT, int P) {
   w.partials = reinterpret_cast<double*>(take((size_t)kNumSMs * 8));
   w.bar = reinterpret_cast<unsigned*>(take((size_t)kMaxLayers * 4));
   w.offmax = reinterpret_cast<unsigned long long*>(take((size_t)kMaxLayers * 2 * 8));
+  int per;
+  w.wpart = det ? reinterpret_cast<float*>(take((size_t)wgrad_splits(M, &per) * nt_slot_floats((int64_t)BN * (Ds + 1)) * sizeof(float))) : nullptr;
   w.bytes = off;
   return w;
 }
@@ -853,9 +863,9 @@ extern "C" {
 size_t dkd_lrkd_workspace_bytes(int n_layers, int64_t B, int n_tok, int Ds, int Dt, int rank, int dtype, int precision) {
   using namespace dkd;
   if (n_layers < 1 || n_layers > kMaxLayers || Dt != kN) return 0;
-  const int P = precision == DKD_PREC_BF16X3 ? 2 : 1;
+  const int P = prec_planes(precision);
   const int PT = dtype == DKD_F32 ? 3 : P;
-  return carve(nullptr, n_layers, B * n_tok, Ds, bn_for_rank(rank), PT, P).bytes;
+  return carve(nullptr, n_layers, B * n_tok, Ds, bn_for_rank(rank), PT, P, prec_deterministic(precision)).bytes;
 }
 
 size_t dkd_lrkd_eigensolve_workspace_bytes(void) { return 1024; }
@@ -886,7 +896,7 @@ int dkd_lrkd_fwdbwd(int n_layers, const void* const* s, const void* const* t, co
   if (rc != DKD_OK) return rc;
   const char* fn = "dkd_lrkd_fwdbwd";
   DKD_REQUIRE(dtype == DKD_F32 || dtype == DKD_BF16, DKD_E_DTYPE, "%s: dtype %d", fn, dtype);
-  DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
+  DKD_REQUIRE(prec_valid(precision), DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
   DKD_REQUIRE(n_layers >= 1 && n_layers <= kMaxLayers, DKD_E_SHAPE, "%s: 1..%d layers", fn, kMaxLayers);
   DKD_REQUIRE(B > 0 && n_tok > 0 && s_off >= 0 && t_off >= 0 && Ts >= s_off + n_tok && Tt >= t_off + n_tok, DKD_E_SHAPE,
               "%s: bad token geometry", fn);
@@ -898,13 +908,13 @@ int dkd_lrkd_fwdbwd(int n_layers, const void* const* s, const void* const* t, co
     DKD_REQUIRE(g_s == nullptr || (((uintptr_t)g_s[l]) & 31) == 0, DKD_E_ALIGN, "%s: g_s[%d] must be 32-byte aligned", fn, l);
   }
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "%s: workspace must be 1024-byte aligned", fn);
-  const int P = precision == DKD_PREC_BF16X3 ? 2 : 1;
+  const int P = prec_planes(precision);
   const int PT = dtype == DKD_F32 ? 3 : P;
   const int BN = bn_for_rank(rank);
   const int64_t M = B * n_tok;
   DKD_REQUIRE(M < (1ll << 31) - 256, DKD_E_SHAPE, "%s: too many rows", fn);
   DKD_REQUIRE(M >= rank, DKD_E_SHAPE, "%s: rank %d exceeds the %lld teacher rows", fn, rank, (long long)M);
-  Workspace ws = carve(workspace, n_layers, M, Ds, BN, PT, P);
+  Workspace ws = carve(workspace, n_layers, M, Ds, BN, PT, P, prec_deterministic(precision));
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   bool want_grads = false;
@@ -1026,12 +1036,18 @@ int dkd_lrkd_fwdbwd(int n_layers, const void* const* s, const void* const* t, co
       if (rc != DKD_OK) return rc;
       rc = launch_fill_ones_tile(ws.ones, st);
       if (rc != DKD_OK) return rc;
-      cudaMemsetAsync(gW, 0, (size_t)rank * Ds * sizeof(float), st);
-      if (gb) cudaMemsetAsync(gb, 0, (size_t)rank * sizeof(float), st);
-      p.ep.D = gW; p.ep.Dcol = gb; p.ep.ldd = Ds; p.ep.alpha = 1.f; p.ep.store = 0; p.ep.rows_valid = rank;
+      const int64_t slot = nt_slot_floats((int64_t)rank * (Ds + 1));   // rank <= BN: fits the carved slots
+      if (ws.wpart) {   // deterministic: each split stores its slot, folded in split order below
+        p.ep.D = ws.wpart; p.ep.Dcol = gb ? ws.wpart + (int64_t)rank * Ds : nullptr; p.ep.store = 1; p.ep.split_stride = slot;
+      } else {
+        cudaMemsetAsync(gW, 0, (size_t)rank * Ds * sizeof(float), st);
+        if (gb) cudaMemsetAsync(gb, 0, (size_t)rank * sizeof(float), st);
+        p.ep.D = gW; p.ep.Dcol = gb; p.ep.store = 0;
+      }
+      p.ep.ldd = Ds; p.ep.alpha = 1.f; p.ep.rows_valid = rank;
       p.ld.ldd = Ds; p.ld.na_tiles = 1; p.ld.b_col0 = 0;
       p.ld.total_row_blocks = (int)((M + Cfg::KROWS - 1) / Cfg::KROWS);
-      nt_make_splits(p.ld.total_row_blocks, kNumSMs, &p.ld.splits, &p.ld.row_blocks_per_split);
+      p.ld.splits = wgrad_splits(M, &p.ld.row_blocks_per_split);
       p.nterms = P == 2 ? 3 : 1;
       const int g3 = min(kNumSMs, p.ld.splits);
       auto kern = gemm_nt_kernel<Cfg, L>;
@@ -1039,6 +1055,10 @@ int dkd_lrkd_fwdbwd(int n_layers, const void* const* s, const void* const* t, co
       kern<<<g3, Cfg::THREADS, Cfg::SMEM, st>>>(p);
       rc = check_launch("dkd_lrkd_fwdbwd: wgrad GEMM");
       if (rc != DKD_OK) return rc;
+      if (ws.wpart) {
+        rc = launch_fold_splits(ws.wpart, p.ld.splits, slot, (int64_t)rank * Ds, gW, gb ? rank : 0, gb, 1.f, st);
+        if (rc != DKD_OK) return rc;
+      }
     }
   }
   return DKD_OK;

@@ -14,6 +14,11 @@
 //   bwd : conv2 wgrad (G^T (*) H) + colsum(G) ; conv2 dgrad (dReLU epilogue) -> DH ; conv1 wgrad + colsum(DH) ;
 //         conv1 dgrad -> dXm (into G) ; masked colsum(dXm) -> g_b_align, g_mask_token ;
 //         g_s = (1-mask) * dXm W_align (row-masked store) ; g_W_align = dXm^T S'
+// Deterministic mode (DKD_PREC_DETERMINISTIC): the two conv wgrads, the align wgrad and the three column sums write
+// per-split (per-CTA) fp32 partials with plain stores into one region appended to the workspace (they run one after
+// another on the stream, so they share it), and each is folded in a fixed order in fp64: conv_wgrad_transpose_kernel
+// for the convolutions, fold_splits_kernel for the align wgrad, fold_rows_kernel for the column sums.  No float atomic
+// is left, and every split count is a function of B alone.
 #include "conv.cuh"
 #include "planes.cuh"
 
@@ -34,9 +39,19 @@ struct Workspace {
   __nv_bfloat16 *S, *X, *H, *G, *DH, *Wa, *Wat, *W1c, *W1d, *W2c, *W2d;
   float *dW1t, *dW2t;
   double* partials;
+  float* wpart;   // deterministic mode only: the weight-gradient / column-sum partials, appended last
   size_t bytes;
 };
-Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
+int conv_wgrad_splits(int64_t B, int slots);
+size_t wpart_bytes(int64_t M, int Ds, int Dt) {
+  const size_t conv = (size_t)conv_wgrad_splits(M / (kHW * kHW), kNumSMs / ConvWgradCfg::CLUSTER) * 9 * Dt * Dt * sizeof(float);
+  int splits, per;   // as the align wgrad launch below
+  nt_make_splits((int)((M + AlignWgradCfg::KROWS - 1) / AlignWgradCfg::KROWS), kNumSMs / (Dt / 128), &splits, &per);
+  const size_t align = (size_t)splits * nt_slot_floats((int64_t)Dt * Ds) * sizeof(float), colsum = colsum_planes_part_bytes(Dt);
+  const size_t m = conv > align ? conv : align;
+  return m > colsum ? m : colsum;
+}
+Workspace carve(void* base, int64_t M, int Ds, int Dt, int P, bool det) {
   Workspace w;
   size_t off = 0;
   auto take = [&](size_t n) { size_t o = off; off = align_up(off + n, 1024); return reinterpret_cast<char*>(base) + o; };
@@ -55,6 +70,7 @@ Workspace carve(void* base, int64_t M, int Ds, int Dt, int P) {
   w.dW1t = reinterpret_cast<float*>(take((size_t)9 * Dt * Dt * 4));
   w.dW2t = reinterpret_cast<float*>(take((size_t)9 * Dt * Dt * 4));
   w.partials = reinterpret_cast<double*>(take((size_t)kNumSMs * sizeof(double)));
+  w.wpart = det ? reinterpret_cast<float*>(take(wpart_bytes(M, Ds, Dt))) : nullptr;
   w.bytes = off;
   return w;
 }
@@ -87,9 +103,18 @@ int run_conv(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParam
   return launch_tn<Cfg, L, E>(p, st, what, grid_out);
 }
 
-// dWt[tap][co][ci] = sum_m G[m, co] * X[m + shift(tap), ci]
-int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, int64_t B, int64_t M, int C, int P, cudaStream_t st,
-                   const char* what) {
+// Items = (tap, ci half) x row splits over the clusters.  The split count is chosen so that the items fill whole waves of
+// `slots` clusters: the former fixed 6 splits gave 324 items on 148 CTAs = 2.19 waves, i.e. a makespan of 3 waves for 2.19
+// waves of work (27 % idle).
+int conv_wgrad_splits(int64_t B, int slots) {
+  return nt_best_splits(NtConvLoader<ConvWgradCfg>::COMBOS_CLUSTER, slots, (int)((B * kHW + 7) / 8), 4, 16);
+}
+
+// dW[co][ci][tap] (PyTorch layout) = sum_m G[m, co] * X[m + shift(tap), ci], through dWt[split][tap][co][ci].  `part` null:
+// the splits add into dWt with float atomics; else (deterministic mode) the split count depends on B alone and each split
+// stores its own slot of `part`, which the transpose kernel folds in split order
+int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, float* part, float* dW, int64_t B, int64_t M, int C, int P,
+                   cudaStream_t st, const char* what) {
   using Cfg = ConvWgradCfg;
   using L = NtConvLoader<Cfg>;
   GemmNtParamsT<Cfg, L> p;
@@ -99,22 +124,27 @@ int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, i
   if (rc != DKD_OK) return rc;
   p.ld.total_hrows = (int)(B * kHW);
   p.ld.total_row_blocks = (p.ld.total_hrows + 7) / 8;
-  // Items = (tap, ci half) x row splits over the clusters.  The split count is chosen so that the items fill whole waves:
-  // the former fixed 6 splits gave 324 items on 148 CTAs = 2.19 waves, i.e. a makespan of 3 waves for 2.19 waves of work
-  // (27 % idle).
   static const int resident = [] {
     auto kern = gemm_nt_kernel<Cfg, L>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
     return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
   }();
-  const int sp = nt_best_splits(L::COMBOS_CLUSTER, resident, p.ld.total_row_blocks, 4, 16);
+  const int sp = conv_wgrad_splits(B, part ? kNumSMs / Cfg::CLUSTER : resident);
   nt_make_splits(p.ld.total_row_blocks, sp, &p.ld.splits, &p.ld.row_blocks_per_split);
-  p.ep.D = dWt; p.ep.Dcol = nullptr; p.ep.ldd = C; p.ep.alpha = 1.f;
+  p.ep.ldd = C; p.ep.alpha = 1.f; p.ep.Dcol = nullptr;
   p.nterms = P == 2 ? 3 : 1;
-  cudaMemsetAsync(dWt, 0, (size_t)9 * C * C * sizeof(float), st);
+  if (part) {
+    p.ep.D = part; p.ep.store = 1; p.ep.split_stride = (int64_t)9 * C * C;   // C % 128 == 0: whole 128-byte slots
+  } else {
+    p.ep.D = dWt;
+    cudaMemsetAsync(dWt, 0, (size_t)9 * C * C * sizeof(float), st);
+  }
+  // each item owns its slot in deterministic mode, so the grid (resident clusters) cannot change a bit
   int grid = min(resident, L::COMBOS_CLUSTER * p.ld.splits) * Cfg::CLUSTER;
   launch_gemm_nt<Cfg, L>(p, grid, st);
-  return check_launch(what);
+  rc = check_launch(what);
+  if (rc != DKD_OK) return rc;
+  return launch_conv_wgrad_transpose(part ? part : dWt, C, part ? p.ld.splits : 1, dW, st);
 }
 
 }  // namespace
@@ -123,11 +153,11 @@ int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, i
 extern "C" {
 
 size_t dkd_masked_generation_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision) {
-  return dkd::carve(nullptr, B * n_tok, Ds, Dt, precision == DKD_PREC_BF16X3 ? 2 : 1).bytes;
+  return dkd::carve(nullptr, B * n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision)).bytes;
 }
 
 size_t dkd_masked_generation_hidden_offset(int64_t B, int n_tok, int Ds, int Dt, int precision) {
-  dkd::Workspace w = dkd::carve(nullptr, B * n_tok, Ds, Dt, precision == DKD_PREC_BF16X3 ? 2 : 1);
+  dkd::Workspace w = dkd::carve(nullptr, B * n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision));
   return (size_t)(reinterpret_cast<char*>(w.H) - static_cast<char*>(nullptr));
 }
 
@@ -142,7 +172,7 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   if (rc != DKD_OK) return rc;
   const char* fn = "dkd_masked_generation_fwdbwd";
   DKD_REQUIRE(dtype == DKD_F32 || dtype == DKD_BF16, DKD_E_DTYPE, "%s: dtype %d", fn, dtype);
-  DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
+  DKD_REQUIRE(prec_valid(precision), DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
   const int n_tok = kHW * kHW;
   DKD_REQUIRE(B > 0 && s_off >= 0 && t_off >= 0 && Ts == s_off + n_tok && Tt == t_off + n_tok, DKD_E_SHAPE,
               "%s: expects %d patch tokens (14x14 grid) after the special tokens", fn, n_tok);
@@ -151,10 +181,10 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
               "%s: null pointer", fn);
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "%s: workspace must be 1024-byte aligned", fn);
   DKD_REQUIRE((((uintptr_t)g_s) & 31) == 0, DKD_E_ALIGN, "%s: g_s must be 32-byte aligned (256-bit stores)", fn);
-  const int P = precision == DKD_PREC_BF16X3 ? 2 : 1;
+  const int P = prec_planes(precision);
   const int64_t M = B * n_tok;
   DKD_REQUIRE(M < (1ll << 31) - 256, DKD_E_SHAPE, "%s: too many rows", fn);
-  Workspace ws = carve(workspace, M, Ds, Dt, P);
+  Workspace ws = carve(workspace, M, Ds, Dt, P, prec_deterministic(precision));
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const bool want_grads = g_s || g_W_align || g_b_align || g_mask_token || g_conv1_w || g_conv1_b || g_conv2_w || g_conv2_b;
@@ -206,13 +236,11 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
 
   // ---- conv2 backward
   if (g_conv2_w) {
-    rc = run_conv_wgrad(ws.G, ws.H, ws.dW2t, B, M, Dt, P, st, "mgd: conv2 wgrad");
-    if (rc != DKD_OK) return rc;
-    rc = launch_conv_wgrad_transpose(ws.dW2t, Dt, g_conv2_w, st);
+    rc = run_conv_wgrad(ws.G, ws.H, ws.dW2t, ws.wpart, g_conv2_w, B, M, Dt, P, st, "mgd: conv2 wgrad");
     if (rc != DKD_OK) return rc;
   }
   if (g_conv2_b) {
-    rc = launch_colsum_planes(ws.G, M, Dt, P, nullptr, g_conv2_b, nullptr, st);
+    rc = launch_colsum_planes(ws.G, M, Dt, P, nullptr, g_conv2_b, nullptr, st, ws.wpart);
     if (rc != DKD_OK) return rc;
   }
   {
@@ -222,13 +250,11 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   }
   // ---- conv1 backward
   if (g_conv1_w) {
-    rc = run_conv_wgrad(ws.DH, ws.X, ws.dW1t, B, M, Dt, P, st, "mgd: conv1 wgrad");
-    if (rc != DKD_OK) return rc;
-    rc = launch_conv_wgrad_transpose(ws.dW1t, Dt, g_conv1_w, st);
+    rc = run_conv_wgrad(ws.DH, ws.X, ws.dW1t, ws.wpart, g_conv1_w, B, M, Dt, P, st, "mgd: conv1 wgrad");
     if (rc != DKD_OK) return rc;
   }
   if (g_conv1_b) {
-    rc = launch_colsum_planes(ws.DH, M, Dt, P, nullptr, g_conv1_b, nullptr, st);
+    rc = launch_colsum_planes(ws.DH, M, Dt, P, nullptr, g_conv1_b, nullptr, st, ws.wpart);
     if (rc != DKD_OK) return rc;
   }
   if (!(g_s || g_W_align || g_b_align || g_mask_token)) return DKD_OK;
@@ -239,7 +265,7 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   }
   // ---- mask-token / alignment backward: masked rows feed mask_token, kept rows feed the Linear
   if (g_b_align || g_mask_token) {
-    rc = launch_colsum_planes(ws.G, M, Dt, P, mask, g_b_align, g_mask_token, st);
+    rc = launch_colsum_planes(ws.G, M, Dt, P, mask, g_b_align, g_mask_token, st, ws.wpart);
     if (rc != DKD_OK) return rc;
   }
   if (g_s) {
@@ -267,8 +293,13 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
     rc = make_plane_tmap(&p.ld.tmB, ws.S, P, M, Ds, Ds, M * Ds, Cfg::KROWS, "mgd S' (wgrad)");
     if (rc != DKD_OK) return rc;
     p.ld.tmOnes = p.ld.tmB;
-    cudaMemsetAsync(g_W_align, 0, (size_t)Dt * Ds * sizeof(float), st);
-    p.ep.D = g_W_align; p.ep.Dcol = nullptr; p.ep.ldd = Ds; p.ep.alpha = 1.f;
+    if (ws.wpart) {   // deterministic: slot per split, folded below
+      p.ep.D = ws.wpart; p.ep.store = 1; p.ep.split_stride = nt_slot_floats((int64_t)Dt * Ds);
+    } else {
+      cudaMemsetAsync(g_W_align, 0, (size_t)Dt * Ds * sizeof(float), st);
+      p.ep.D = g_W_align;
+    }
+    p.ep.Dcol = nullptr; p.ep.ldd = Ds; p.ep.alpha = 1.f;
     p.ld.ldd = Ds; p.ld.na_tiles = Dt / 128; p.ld.b_col0 = 0;
     p.ld.total_row_blocks = (int)((M + Cfg::KROWS - 1) / Cfg::KROWS);
     nt_make_splits(p.ld.total_row_blocks, kNumSMs / p.ld.na_tiles, &p.ld.splits, &p.ld.row_blocks_per_split);
@@ -279,6 +310,10 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
     kern<<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(p);
     rc = check_launch("mgd: align wgrad");
     if (rc != DKD_OK) return rc;
+    if (ws.wpart) {
+      rc = launch_fold_splits(ws.wpart, p.ld.splits, p.ep.split_stride, (int64_t)Dt * Ds, g_W_align, 0, nullptr, 1.f, st);
+      if (rc != DKD_OK) return rc;
+    }
   }
   return DKD_OK;
 }

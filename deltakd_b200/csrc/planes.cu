@@ -76,12 +76,61 @@ __global__ void conv_weight_to_planes_kernel(const float* __restrict__ W, int C,
   }
 }
 
-// dWt[tap][co][ci] fp32 -> dW[co][ci][tap] (PyTorch conv weight layout)
-__global__ void conv_wgrad_transpose_kernel(const float* __restrict__ dWt, int C, float* __restrict__ dW) {
+// dWt[split][tap][co][ci] fp32 -> dW[co][ci][tap] (PyTorch conv weight layout).  splits = 1: a gather in output order.
+// splits > 1 (deterministic mode): the splits are added in split order in fp64, threads walking the source order so that
+// the `splits` reads per element are coalesced and only its one store is strided.
+__global__ void conv_wgrad_transpose_kernel(const float* __restrict__ dWt, int C, int splits, float* __restrict__ dW) {
   const int total = C * C * 9;
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
-    const int tap = idx % 9, ci = (idx / 9) % C, co = idx / (9 * C);
-    dW[idx] = dWt[((int64_t)tap * C + co) * C + ci];
+    if (splits == 1) {
+      const int tap = idx % 9, ci = (idx / 9) % C, co = idx / (9 * C);
+      dW[idx] = dWt[((int64_t)tap * C + co) * C + ci];
+    } else {
+      const int ci = idx % C, co = (idx / C) % C, tap = idx / (C * C);
+      double a = dWt[idx];
+#pragma unroll 4
+      for (int s = 1; s < splits; ++s) a += (double)dWt[(int64_t)s * total + idx];
+      dW[((int64_t)co * C + ci) * 9 + tap] = (float)a;
+    }
+  }
+}
+
+// out0[i] = alpha * sum_s part[s * stride + i] (i < n0), out1[i - n0] likewise (n0 <= i < n0 + n1): the per-split slots
+// of a deterministic split-K product, added in slot order in fp64.  Null outputs are skipped.
+__global__ void fold_splits_kernel(const float* __restrict__ part, int splits, int64_t stride, int64_t n0, float* __restrict__ out0,
+                                   int64_t n1, float* __restrict__ out1, float alpha) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n0 + n1; i += (int64_t)gridDim.x * blockDim.x) {
+    float* out = i < n0 ? (out0 ? out0 + i : nullptr) : (out1 ? out1 + (i - n0) : nullptr);
+    if (out == nullptr) continue;
+    double a = part[i];
+#pragma unroll 4
+    for (int s = 1; s < splits; ++s) a += (double)part[(int64_t)s * stride + i];
+    *out = (float)(a * (double)alpha);
+  }
+}
+
+// Column sums' fold: many partial rows (up to 592 per-CTA rows) over few columns (2N).  One CTA per 32 columns: warp w
+// adds rows w, w + 32, w + 64, ... in increasing order (fp64), then warp 0 adds the 32 warp sums in warp order.  The
+// order depends on `rows` only, so the result is deterministic, and each thread's chain is rows / 32 loads long instead
+// of `rows` (fold_splits_kernel's one-thread-per-output form).
+constexpr int kFoldRowsWarps = 32;
+__global__ void __launch_bounds__(kFoldRowsWarps * 32) fold_rows_kernel(const float* __restrict__ part, int rows, int ncols, int64_t n0,
+                                                                       float* __restrict__ out0, float* __restrict__ out1) {
+  __shared__ double s_sum[kFoldRowsWarps][33];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int col = blockIdx.x * 32 + lane;
+  double a = 0.0;
+  if (col < ncols) {
+#pragma unroll 4
+    for (int r = warp; r < rows; r += kFoldRowsWarps) a += (double)part[(int64_t)r * ncols + col];
+  }
+  s_sum[warp][lane] = a;
+  __syncthreads();
+  if (warp == 0 && col < ncols) {
+    double t = s_sum[0][lane];
+    for (int w = 1; w < kFoldRowsWarps; ++w) t += s_sum[w][lane];
+    float* out = col < n0 ? (out0 ? out0 + col : nullptr) : (out1 ? out1 + (col - n0) : nullptr);
+    if (out) *out = (float)t;
   }
 }
 
@@ -90,11 +139,13 @@ __global__ void conv_wgrad_transpose_kernel(const float* __restrict__ dWt, int C
 // One HBM pass: a thread owns 8 adjacent columns (16-byte loads of both planes), the CTA's row lanes stride over a
 // contiguous block of rows with two rows in flight, lanes are combined in shared memory and each CTA issues one
 // atomicAdd per column (592 CTAs x N atomics; the former one-row-per-CTA-iteration form took 85-95 us per call for
-// 77-154 MB — 10 % of the bf16 MGD step).
+// 77-154 MB — 10 % of the bf16 MGD step).  With `part` (deterministic mode) the CTA stores its two sums as row
+// part[cta][2][N] instead, and fold_rows_kernel adds the rows in a fixed order.
 constexpr int kColsumThreads = 256;
 __global__ void __launch_bounds__(kColsumThreads) colsum_planes_kernel(const __nv_bfloat16* __restrict__ X, int64_t M, int N, int P,
                                                                        const float* __restrict__ mask, int64_t rows_per_cta,
-                                                                       float* __restrict__ out_keep, float* __restrict__ out_masked) {
+                                                                       float* __restrict__ out_keep, float* __restrict__ out_masked,
+                                                                       float* __restrict__ part) {
   extern __shared__ float s_cs[];   // [2][RL][N]
   const int G = N >> 3, RL = kColsumThreads / G;
   const int cg = threadIdx.x % G, rl = threadIdx.x / G;
@@ -148,7 +199,8 @@ __global__ void __launch_bounds__(kColsumThreads) colsum_planes_kernel(const __n
     if (out == nullptr) continue;
     float a = 0.f;
     for (int q = 0; q < RL; ++q) a += s_cs[(which * RL + q) * N + c];
-    atomicAdd(out + c, a);
+    if (part) part[(int64_t)blockIdx.x * 2 * N + k] = a;
+    else atomicAdd(out + c, a);
   }
 }
 
@@ -202,17 +254,27 @@ int launch_conv_weight_to_planes(const float* W, int C, int P, __nv_bfloat16* Wc
   return check_launch("conv_weight_to_planes");
 }
 
-int launch_conv_wgrad_transpose(const float* dWt, int C, float* dW, cudaStream_t st) {
-  conv_wgrad_transpose_kernel<<<kNumSMs * 4, 256, 0, st>>>(dWt, C, dW);
+int launch_conv_wgrad_transpose(const float* dWt, int C, int splits, float* dW, cudaStream_t st) {
+  conv_wgrad_transpose_kernel<<<kNumSMs * 4, 256, 0, st>>>(dWt, C, splits, dW);
   return check_launch("conv_wgrad_transpose");
 }
 
+int launch_fold_splits(const float* part, int splits, int64_t stride, int64_t n0, float* out0, int64_t n1, float* out1, float alpha,
+                       cudaStream_t st) {
+  int64_t blocks = (n0 + n1 + 255) / 256;
+  if (blocks > (int64_t)kNumSMs * 8) blocks = (int64_t)kNumSMs * 8;
+  fold_splits_kernel<<<(unsigned)blocks, 256, 0, st>>>(part, splits, stride, n0, out0, n1, out1, alpha);
+  return check_launch("fold_splits");
+}
+
+size_t colsum_planes_part_bytes(int N) { return (size_t)kNumSMs * 4 * 2 * N * sizeof(float); }
+
 int launch_colsum_planes(const __nv_bfloat16* X, int64_t M, int N, int P, const float* mask, float* out_keep, float* out_masked,
-                         cudaStream_t st) {
+                         cudaStream_t st, float* part) {
   DKD_REQUIRE(N % 8 == 0 && N / 8 <= kColsumThreads, DKD_E_SHAPE, "colsum_planes: N");
   DKD_REQUIRE((((uintptr_t)X) & 15) == 0, DKD_E_ALIGN, "colsum_planes: 16-byte alignment");
-  if (out_keep) cudaMemsetAsync(out_keep, 0, (size_t)N * sizeof(float), st);
-  if (out_masked) cudaMemsetAsync(out_masked, 0, (size_t)N * sizeof(float), st);
+  if (!part && out_keep) cudaMemsetAsync(out_keep, 0, (size_t)N * sizeof(float), st);
+  if (!part && out_masked) cudaMemsetAsync(out_masked, 0, (size_t)N * sizeof(float), st);
   const int RL = kColsumThreads / (N / 8);
   int64_t blocks = (M + 2 * RL - 1) / (2 * RL);          // at least two rows per row lane
   if (blocks > (int64_t)kNumSMs * 4) blocks = (int64_t)kNumSMs * 4;
@@ -220,8 +282,11 @@ int launch_colsum_planes(const __nv_bfloat16* X, int64_t M, int N, int P, const 
   const int64_t rows_per_cta = (M + blocks - 1) / blocks;
   blocks = (M + rows_per_cta - 1) / rows_per_cta;
   const size_t smem = (size_t)2 * RL * N * sizeof(float);
-  colsum_planes_kernel<<<(unsigned)blocks, kColsumThreads, smem, st>>>(X, M, N, P, mask, rows_per_cta, out_keep, out_masked);
-  return check_launch("colsum_planes");
+  colsum_planes_kernel<<<(unsigned)blocks, kColsumThreads, smem, st>>>(X, M, N, P, mask, rows_per_cta, out_keep, out_masked, part);
+  int rc = check_launch("colsum_planes");
+  if (rc != DKD_OK || !part) return rc;
+  fold_rows_kernel<<<(2 * N + 31) / 32, kFoldRowsWarps * 32, 0, st>>>(part, (int)blocks, 2 * N, N, out_keep, out_masked);
+  return check_launch("colsum_planes: fold");
 }
 
 int launch_fill_ones_tile(__nv_bfloat16* ones, cudaStream_t st) {

@@ -441,9 +441,10 @@ struct Workspace {
   float *A, *nx, *ny, *C, *eps;
   int* n_eps;
   double* partials;
+  float* wpart;   // deterministic mode: per-split weight-gradient slots (align_wgrad), appended last
   size_t bytes;
 };
-Workspace carve(void* base, int64_t B, int Ds, int Dt, int P) {
+Workspace carve(void* base, int64_t B, int Ds, int Dt, int P, bool det) {
   Workspace w;
   const int64_t M = B * kTok;
   size_t off = 0;
@@ -463,6 +464,7 @@ Workspace carve(void* base, int64_t B, int Ds, int Dt, int P) {
   w.eps = reinterpret_cast<float*>(take((size_t)B * kMaxEps * 4));
   w.n_eps = reinterpret_cast<int*>(take((size_t)B * 4));
   w.partials = reinterpret_cast<double*>(take((size_t)B * 3 * sizeof(double)));
+  w.wpart = det ? reinterpret_cast<float*>(take(align_wgrad_part_bytes(B * kTok, Ds, Dt, P))) : nullptr;
   w.bytes = off;
   return w;
 }
@@ -482,7 +484,7 @@ extern "C" {
 
 size_t dkd_wass_sinkhorn_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision) {
   (void)n_tok;
-  return dkd::carve(nullptr, B, Ds, Dt, precision == DKD_PREC_BF16X3 ? 2 : 1).bytes;
+  return dkd::carve(nullptr, B, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision)).bytes;
 }
 
 int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* W, const float* bias, int64_t B, int Ts, int s_off, int Tt,
@@ -493,7 +495,7 @@ int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* W, const
   if (rc != DKD_OK) return rc;
   const char* fn = "dkd_wass_sinkhorn_fwdbwd";
   DKD_REQUIRE(dtype == DKD_F32 || dtype == DKD_BF16, DKD_E_DTYPE, "%s: dtype %d", fn, dtype);
-  DKD_REQUIRE(precision == DKD_PREC_BF16 || precision == DKD_PREC_BF16X3, DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
+  DKD_REQUIRE(prec_valid(precision), DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
   DKD_REQUIRE(n_tok == kTok, DKD_E_SHAPE, "%s: built for %d patch tokens per sample, got %d", fn, kTok, n_tok);
   DKD_REQUIRE(B > 0 && s_off >= 0 && t_off >= 0 && Ts >= s_off + n_tok && Tt >= t_off + n_tok, DKD_E_SHAPE, "%s: bad token geometry", fn);
   DKD_REQUIRE(Ds == 192 && Dt == kD, DKD_E_SHAPE, "%s: built for widths 192 -> 384, got %d -> %d", fn, Ds, Dt);
@@ -501,9 +503,9 @@ int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* W, const
   DKD_REQUIRE((((uintptr_t)workspace) & 1023) == 0, DKD_E_ALIGN, "%s: workspace must be 1024-byte aligned", fn);
   DKD_REQUIRE((((uintptr_t)s | (uintptr_t)t | (uintptr_t)g_s) & 31) == 0, DKD_E_ALIGN, "%s: s, t and g_s must be 32-byte aligned (256-bit accesses)", "dkd_wass_sinkhorn_fwdbwd");
   DKD_REQUIRE(B * 6 < (1ll << 24), DKD_E_SHAPE, "%s: too many samples", fn);
-  const int P = precision == DKD_PREC_BF16X3 ? 2 : 1;
+  const int P = prec_planes(precision);
   const int64_t M = B * kTok;
-  Workspace ws = carve(workspace, B, Ds, Dt, P);
+  Workspace ws = carve(workspace, B, Ds, Dt, P, prec_deterministic(precision));
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const bool want_grads = g_s || g_W || g_b;
@@ -599,7 +601,7 @@ int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* W, const
   }
   if (g_W || g_b) {
     DKD_REQUIRE(g_W != nullptr, DKD_E_UNSUPPORTED, "%s: g_b without g_W is not supported", fn);
-    rc = align_wgrad(ws.G, ws.S, ws.ones, g_W, g_b, M, Ds, Dt, P, 1.f, st, "dkd_wass_sinkhorn_fwdbwd: wgrad GEMM");
+    rc = align_wgrad(ws.G, ws.S, ws.ones, g_W, g_b, M, Ds, Dt, P, 1.f, st, "dkd_wass_sinkhorn_fwdbwd: wgrad GEMM", 0, ws.wpart);
     if (rc != DKD_OK) return rc;
   }
   return DKD_OK;

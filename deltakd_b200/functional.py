@@ -246,6 +246,20 @@ def _precision_for(t: torch.Tensor) -> int:
     return _lib.PREC_BF16X3 if mode == "bf16x3" else _lib.PREC_BF16
 
 
+def _deterministic() -> bool:
+    """True when the feature losses run in their deterministic mode (DKD_PREC_DETERMINISTIC): bit-reproducible weight,
+    bias and mask-token gradients.  It follows torch state, read at every call: torch.use_deterministic_algorithms(True),
+    or torch.backends.cudnn.deterministic = True, which the reference trainer sets to pin the cuDNN convolutions that
+    the masked-generation kernels replace."""
+    return torch.are_deterministic_algorithms_enabled() or bool(torch.backends.cudnn.deterministic)
+
+
+def _grad_precision_for(t: torch.Tensor) -> int:
+    """`precision` of a gradient-bearing feature entry point: _precision_for, plus the deterministic bit when requested."""
+    prec = _precision_for(t)
+    return prec | _lib.PREC_DETERMINISTIC if _deterministic() else prec
+
+
 def _scratch(device: torch.device, tag: str, nbytes: int) -> torch.Tensor:
     """Uninitialised, 1024-byte aligned scratch cached per (device, stream, tag)."""
     key = (device.index, _stream(), "scratch:" + tag)
@@ -308,7 +322,7 @@ class _AlignMseLayers(torch.autograd.Function):
             _, Tt, Dt = t.shape
             n_tok = Ts - s_off
             dt = _dtype_code(s)
-            prec = _precision_for(s)
+            prec = _grad_precision_for(s)
             g_s, g_W, g_b = outs[i]
             nbytes = getattr(_lib.lib, entry + "_workspace_bytes")(B, n_tok, Ds, Dt, prec)
             with torch.cuda.stream(main if (i == 0 or not multi) else sides[i - 1]):
@@ -424,7 +438,7 @@ class _MaskedGeneration(torch.autograd.Function):
         B, Ts, Ds = s.shape
         _, Tt, Dt = t.shape
         dev = s.device
-        prec = _precision_for(s)
+        prec = _grad_precision_for(s)
         need = ctx.needs_input_grad[6:]
         g_s = torch.empty_like(s) if need[0] else None
         outs = [g_s]
@@ -438,7 +452,7 @@ class _MaskedGeneration(torch.autograd.Function):
                   _ptr(c1w), _ptr(c1b), _ptr(c2w), _ptr(c2b), B, Ts, s_off, Tt, t_off, Ds, Dt, _dtype_code(s), prec,
                   float(scale), *[_ptr(o) for o in outs], _ptr(loss), _ptr(ws), ws.numel(), _stream())
         if probe is not None:   # verification hook: the hidden activations (ReLU gate) the backward pass used
-            P = 2 if prec == _lib.PREC_BF16X3 else 1
+            P = 2 if (prec & ~_lib.PREC_DETERMINISTIC) == _lib.PREC_BF16X3 else 1
             M = B * (Ts - s_off)
             off = _lib.lib.dkd_masked_generation_hidden_offset(B, Ts - s_off, Ds, Dt, prec)
             probe["hidden"] = ws[off:off + P * M * Dt * 2].view(torch.bfloat16).view(P, B, Ts - s_off, Dt).clone()
@@ -584,7 +598,7 @@ class _LrkdLayers(torch.autograd.Function):
         B, Ts, Ds = s0.shape
         _, Tt, Dt = t0.shape
         n_tok = Ts - s_off
-        prec = _precision_for(s0)
+        prec = _grad_precision_for(s0)
         dt = _dtype_code(s0)
         g_s = [torch.empty_like(s) if ctx.needs_input_grad[6 + i] else None for i, s in enumerate(s_list)]
         need_w = [ctx.needs_input_grad[6 + 2 * n_layers + i] for i in range(n_layers)]

@@ -50,8 +50,14 @@ enum {
 /* tensor-core arithmetic of the dense contractions */
 enum {
   DKD_PREC_BF16 = 0,  /* one bf16 tcgen05 pass, fp32 accumulate                                  */
-  DKD_PREC_BF16X3 = 1 /* hi/lo bf16 split, 3 passes (hi*hi + hi*lo + lo*hi): ~2^-16 relative,   */
-                      /* the mode that meets the fp32 parity gates                              */
+  DKD_PREC_BF16X3 = 1, /* hi/lo bf16 split, 3 passes (hi*hi + hi*lo + lo*hi): ~2^-16 relative,  */
+                       /* the mode that meets the fp32 parity gates                             */
+  /* OR'ed into `precision` of the gradient-bearing feature entry points (align_mse, align_nmse, wass_l1,
+   * wass_sinkhorn, masked_generation, lrkd: *_workspace_bytes, *_fwdbwd, and dkd_masked_generation_hidden_offset):
+   * every gradient is bit-reproducible.  Split-K weight gradients and column sums store one fp32 partial per split
+   * (per CTA) into the workspace and a fold kernel adds them in split order in fp64; split counts and grids depend on
+   * the shapes only.  The workspace grows by those partial regions (appended after the others). */
+  DKD_PREC_DETERMINISTIC = 0x100
 };
 
 DKD_API int dkd_version(void);
@@ -122,7 +128,8 @@ DKD_API int dkd_scale_if_not_one(void* x, int64_t n, void* x2, int64_t n2, int d
  * mimicking term (loss.py:277-289; scale = alpha_vitkd/B).
  *   s [B,Ts,Ds], t [B,Tt,Dt] : `dtype`, contiguous, special tokens included (consumed in place)
  *   W [Dt,Ds], bias [Dt], g_W, g_b, loss : fp32 ;  g_s : `dtype`  (any g_* may be NULL)
- *   precision : DKD_PREC_BF16 | DKD_PREC_BF16X3 (tcgen05 bf16 passes, fp32 accumulate in TMEM)
+ *   precision : DKD_PREC_BF16 | DKD_PREC_BF16X3 (tcgen05 bf16 passes, fp32 accumulate in TMEM), optionally
+ *               | DKD_PREC_DETERMINISTIC (bit-reproducible g_W / g_b; pass the same value to the workspace query)
  *   workspace : >= dkd_align_mse_workspace_bytes(...) bytes, 1024-byte aligned, contents don't matter
  * Built for Ds = 192 with Dt = 384 (DeiT-Tiny -> DeiT-Small) or Dt = 768 (DeiT-Tiny -> DeiT-Base); any other pair
  * returns DKD_E_SHAPE.
@@ -201,7 +208,8 @@ DKD_API int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* 
  */
 DKD_API size_t dkd_masked_generation_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision);
 /* Byte offset, inside the workspace, of the generator's hidden activations h = relu(conv1(x_m)) as bf16 planes
- * [P][B*196][Dt] (P = 2 hi/lo planes for DKD_PREC_BF16X3, else 1).  They stay valid after dkd_masked_generation_fwdbwd
+ * [P][B*196][Dt] (P = 2 hi/lo planes for DKD_PREC_BF16X3, else 1; DKD_PREC_DETERMINISTIC does not move them).  They
+ * stay valid after dkd_masked_generation_fwdbwd
  * returns: verification code reads the ReLU gate the backward pass used from them (h != 0), because the gradient of
  * F.relu (models.py:150) is discontinuous at 0 and parity of the gradients is only defined given the same gate. */
 DKD_API size_t dkd_masked_generation_hidden_offset(int64_t B, int n_tok, int Ds, int Dt, int precision);
