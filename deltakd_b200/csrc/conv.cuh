@@ -1,36 +1,54 @@
-// 3x3 / pad 1 convolution on the 14x14 token grid as implicit GEMM on tcgen05 (sm_100a).
-// The [B, 196, C] token layout is NHWC, so no permute is needed (the reference permutes to NCHW,
-// model/loss.py:444).  Activations are bf16 plane tensors [P][B*196][C]; viewed through a 4-D tensor map
-// {c, w, hb, plane} (hb = b*14 + h) a TMA box {64, 14, 1, 1} is one image row of 64 channels, and the
-// zero padding comes for free: the w coordinate starts at dx-1 (out-of-bounds columns are zero-filled by
-// TMA) and rows that fall outside their image are requested at an out-of-bounds hb coordinate.
+// 3x3 / pad 1 convolution on the HW x HW token grid (HW = 14: 224-px inputs, HW = 24: 384-px inputs, patch 16) as implicit
+// GEMM on tcgen05 (sm_100a).  The [B, HW*HW, C] token layout is NHWC, so no permute is needed (the reference permutes to
+// NCHW, model/loss.py:444).  Activations are bf16 plane tensors [P][B*HW*HW][C]; viewed through a 4-D tensor map
+// {c, w, hb, plane} (hb = b*HW + h) a TMA box {64, HW, 1, 1} is one image row of 64 channels, and the zero padding comes
+// for free: the w coordinate starts at dx-1 (out-of-bounds columns are zero-filled by TMA) and rows that fall outside
+// their image are requested at an out-of-bounds hb coordinate.
 //
-//   forward / dgrad  (gemm_tn): tile = 9 image rows = 126 pixels x 384 channels; K walks 9 taps x 6 chunks.
+//   forward / dgrad  (gemm_tn): tile = 128 / HW whole image rows (9 x 14 = 126, 5 x 24 = 120 pixels) x 384 channels;
+//                     K walks 9 taps x 6 chunks.  Accumulator rows >= TILE_M are dead.
 //                     out[m, co] = sum_{tap, ci} X[m + shift(tap), ci] * Wc[co, tap*C + ci]
-//   wgrad            (gemm_nt): dW[tap][co][ci] += sum_m G[m, co] * X[m + shift(tap), ci], K block = 8 image rows.
+//   wgrad            (gemm_nt): dW[tap][co][ci] += sum_m G[m, co] * X[m + shift(tap), ci], K block = conv_wgrad_rows(HW)
+//                     whole image rows (8 x 14 = 112, 4 x 24 = 96 pixels).
 #pragma once
 #include "epilogues.cuh"
 #include "gemm_nt.cuh"
 
 namespace dkd {
 
-constexpr int kHW = 14;            // token grid side
-constexpr int kRowBytes = kHW * 128;  // one image row of 64 bf16 channels in shared memory
+// one image row of 64 bf16 channels in shared memory
+template <int HW>
+constexpr int conv_row_bytes() { return HW * 128; }
+
+// image rows per forward / dgrad tile: as many whole rows as fit the 128-row UMMA tile
+template <int HW>
+constexpr int conv_tile_m() { return 128 / HW * HW; }
+
+// image rows per wgrad K block: the most whole rows whose pixel count is a multiple of the UMMA K step (16) and at most
+// 112 (the block that keeps three 5-box stages in shared memory).  Whole rows, so the padding test is per TMA box.
+template <int HW>
+constexpr int conv_wgrad_rows() {
+  int best = 0;
+  for (int r = 1; r * HW <= 112; ++r)
+    if (r * HW % 16 == 0) best = r;
+  return best;
+}
 
 struct ConvLoaderParams {
-  CUtensorMap tmX;   // 4-D {C, 14, B*14, P}, box {64, 14, 1, 1}
+  CUtensorMap tmX;   // 4-D {C, HW, B*HW, P}, box {64, HW, 1, 1}
   CUtensorMap tmW;   // 3-D {9*C, C_out, P}, box {64, 192, 1}
-  int total_hrows;   // B * 14
+  int total_hrows;   // B * HW
   int nterms;        // 1 | 3
 };
 
-template <class Cfg>
+template <class Cfg, int HW>
 struct ConvRowsLoader {
   using Params = ConvLoaderParams;
-  static constexpr int ROWS = Cfg::TILE_M / kHW;  // image rows per tile (9)
-  static constexpr int KB = 54;                   // 9 taps x 6 channel chunks (C = 384)
+  static constexpr int kRowBytes = conv_row_bytes<HW>();
+  static constexpr int ROWS = Cfg::TILE_M / HW;  // image rows per tile (9 at HW = 14, 5 at HW = 24)
+  static constexpr int KB = 54;                  // 9 taps x 6 channel chunks (C = 384)
   static constexpr uint32_t TX_BYTES = ROWS * kRowBytes + Cfg::B_BYTES;
-  static_assert(Cfg::TILE_M % kHW == 0 && Cfg::BN == 384, "conv tile");
+  static_assert(Cfg::TILE_M == conv_tile_m<HW>() && Cfg::BN == 384, "conv tile");
   static __device__ __forceinline__ int num_k_iters(const Params& p) { return KB * p.nterms; }
   static __device__ __forceinline__ void prefetch(const Params& p) {
     sm100::tma_prefetch_desc(&p.tmX);
@@ -50,8 +68,8 @@ struct ConvRowsLoader {
 #pragma unroll
     for (int rr = 0; rr < ROWS; ++rr) {
       const int hb = mt * ROWS + rr;
-      const int sh = hb % kHW + dy - 1;
-      const bool ok = sh >= 0 && sh < kHW && hb < p.total_hrows;
+      const int sh = hb % HW + dy - 1;
+      const bool ok = sh >= 0 && sh < HW && hb < p.total_hrows;
       sm100::tma_load_4d(sA + rr * kRowBytes, &p.tmX, bar, cb * 64, dx - 1, ok ? hb + dy - 1 : -4, pa);
     }
     sm100::tma_load_3d_mc(sB + (size_t)crank * W_ROWS * 128, &p.tmW, bar, tap * 384 + cb * 64, nt * Cfg::BN + crank * W_ROWS, pb,
@@ -138,19 +156,21 @@ struct ConvEpi {
   }
 };
 
-// ---- wgrad loader (gemm_nt): A = G planes [P][M][C] (3-D map, box {64, 112, 1}), B = shifted X rows ----
+// ---- wgrad loader (gemm_nt): A = G planes [P][M][C] (3-D map, box {64, KROWS, 1}), B = shifted X rows ----
 struct NtConvParams {
-  CUtensorMap tmG;   // 3-D {C, M, P}, box {64, 112, 1}
-  CUtensorMap tmX;   // 4-D {C, 14, B*14, P}, box {64, 14, 1, 1}
+  CUtensorMap tmG;   // 3-D {C, M, P}, box {64, KROWS, 1}
+  CUtensorMap tmX;   // 4-D {C, HW, B*HW, P}, box {64, HW, 1, 1}
   int splits, row_blocks_per_split, total_row_blocks, total_hrows;
 };
-template <class Cfg>
+template <class Cfg, int HW>
 struct NtConvLoader {
   using Params = NtConvParams;
   using Item = NtItem;
   static constexpr int COMBOS_CLUSTER = 9 * 2;   // tap x ci half (192); the cluster's 3 CTAs are the co tiles (128)
+  static constexpr int kRowBytes = conv_row_bytes<HW>();
+  static constexpr int RB_ROWS = conv_wgrad_rows<HW>();   // image rows per K block (8 at HW = 14, 4 at HW = 24)
   static constexpr uint32_t TX_BYTES = Cfg::STAGE_BYTES;
-  static_assert(Cfg::KROWS == 8 * kHW && Cfg::NB_BOXES == 3 && !Cfg::ONES, "conv wgrad stage = 8 image rows x 192 channels");
+  static_assert(Cfg::KROWS == RB_ROWS * HW && Cfg::NB_BOXES == 3 && !Cfg::ONES, "conv wgrad stage = RB_ROWS image rows x 192 channels");
   static_assert(Cfg::CLUSTER == 3, "a cluster = the 3 output-channel tiles");
   static __device__ __forceinline__ int num_items(const Params& p) { return COMBOS_CLUSTER * p.splits; }
   static __device__ __forceinline__ void prefetch(const Params& p) {
@@ -181,10 +201,10 @@ struct NtConvLoader {
     sm100::tma_load_3d(a, &p.tmG, bar, it.a_col0, rb * Cfg::KROWS, pa);
     sm100::tma_load_3d(a + Cfg::BOX_BYTES, &p.tmG, bar, it.a_col0 + 64, rb * Cfg::KROWS, pa);
 #pragma unroll
-    for (int rr = 0; rr < 8; ++rr) {
-      const int hb = rb * 8 + rr;
-      const int sh = hb % kHW + dy - 1;
-      const bool ok = sh >= 0 && sh < kHW && hb < p.total_hrows;
+    for (int rr = 0; rr < RB_ROWS; ++rr) {
+      const int hb = rb * RB_ROWS + rr;
+      const int sh = hb % HW + dy - 1;
+      const bool ok = sh >= 0 && sh < HW && hb < p.total_hrows;
       const int coord = ok ? hb + dy - 1 : -4;
       sm100::tma_load_4d_mc(b + (size_t)crank * Cfg::BOX_BYTES + rr * kRowBytes, &p.tmX, bar, it.b_col0 + crank * 64, dx - 1, coord, pb,
                             (uint16_t)0x7);
@@ -192,11 +212,11 @@ struct NtConvLoader {
   }
 };
 
-// host: 4-D activation map {C, 14, B*14, P} over planes [P][B*196][C]
-inline int make_image_tmap(CUtensorMap* out, const void* base, int64_t B, int C, int P, const char* what) {
-  const uint64_t dims[4] = {(uint64_t)C, (uint64_t)kHW, (uint64_t)(B * kHW), (uint64_t)P};
-  const uint64_t strides[3] = {(uint64_t)C * 2, (uint64_t)C * kHW * 2, (uint64_t)B * 196 * C * 2};
-  const uint32_t box[4] = {64, (uint32_t)kHW, 1, 1};
+// host: 4-D activation map {C, HW, B*HW, P} over planes [P][B*HW*HW][C]
+inline int make_image_tmap(CUtensorMap* out, const void* base, int64_t B, int HW, int C, int P, const char* what) {
+  const uint64_t dims[4] = {(uint64_t)C, (uint64_t)HW, (uint64_t)(B * HW), (uint64_t)P};
+  const uint64_t strides[3] = {(uint64_t)C * 2, (uint64_t)C * HW * 2, (uint64_t)B * HW * HW * C * 2};
+  const uint32_t box[4] = {64, (uint32_t)HW, 1, 1};
   return make_tmap_bf16(out, base, 4, dims, strides, box, what);
 }
 

@@ -1,11 +1,13 @@
 // Masked generative distillation core, forward + backward:
 //     x   = align(s[:, s_off:])                       Linear(Ds -> Dt)
 //     x_m = where(mask, mask_token, x)
-//     h   = relu(conv3x3(x_m; W1, b1)) ; g = conv3x3(h; W2, b2)      on the 14x14 token grid, pad 1
+//     h   = relu(conv3x3(x_m; W1, b1)) ; g = conv3x3(h; W2, b2)      on the HW x HW token grid, pad 1
 //     loss += scale * sum( mask * (g - t[:, t_off:])^2 )
 // Reference: mgd_loss (model/loss.py:422-451), saliency_mgd_loss (:335-360), curkd_loss late phase (:394-420)
 // and the ViTKD generation term (:291-310) — they differ only in how `mask` is chosen and in `scale`.
 // The reference's cat/gather with ids_restore equals where(mask, mask_token, x) (SURVEY.md A.4).
+// The grid side HW is 14 (196 patch tokens, 224-px inputs) or 24 (576 tokens, 384-px inputs); it only changes the
+// convolutions' tiling (conv.cuh), so each generator convolution is instantiated for both and picked from n_tok.
 //
 // Every contraction runs on tcgen05 (gemm_tn / gemm_nt skeletons); activations travel between the
 // GEMMs as bf16 hi/lo planes.  Launch sequence (one stream, no host sync):
@@ -26,11 +28,13 @@ namespace dkd {
 namespace {
 
 using AlignCfg = GemmCfg<192, 1, 4, 2, 128, 1, 8>;   // X tile 128 x 192 (K = 192), 8 epilogue warps
-// 9 image rows x 384 channels, K = 9 x 384, 8 epilogue warps; clusters of 2 CTAs with the weight block multicast
-using ConvCfg = GemmCfg<384, 2, 3, 1, 126, 1, 8, 2>;
+// 128 / HW image rows x 384 channels, K = 9 x 384, 8 epilogue warps; clusters of 2 CTAs with the weight block multicast
+template <int HW>
+using ConvCfg = GemmCfg<384, 2, 3, 1, conv_tile_m<HW>(), 1, 8, 2>;
 using DalignCfg = GemmCfg<192, 1, 4, 2, 128, 1, 8>;  // g_s tile 128 x 192 (K = 384)
-// dW tile 128(co) x 192(ci), 8 image rows per stage; 3-CTA clusters with the shifted-X block multicast
-using ConvWgradCfg = GemmNtCfg<3, false, 192, 0, 3, 112, false, 1, 3>;
+// dW tile 128(co) x 192(ci), conv_wgrad_rows<HW>() image rows per stage; 3-CTA clusters with the shifted-X block multicast
+template <int HW>
+using ConvWgradCfg = GemmNtCfg<3, false, 192, 0, 3, conv_wgrad_rows<HW>() * HW, false, 1, 3>;
 using AlignWgradCfg = GemmNtCfg<3, false, 192, 0, 4>;      // g_W_align tile 128 x 192
 
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -42,17 +46,26 @@ struct Workspace {
   float* wpart;   // deterministic mode only: the weight-gradient / column-sum partials, appended last
   size_t bytes;
 };
+
+// grid side of a supported patch-token count, 0 for any other
+int grid_side(int n_tok) { return n_tok == 14 * 14 ? 14 : n_tok == 24 * 24 ? 24 : 0; }
+
+template <int HW>
 int conv_wgrad_splits(int64_t B, int slots);
-size_t wpart_bytes(int64_t M, int Ds, int Dt) {
-  const size_t conv = (size_t)conv_wgrad_splits(M / (kHW * kHW), kNumSMs / ConvWgradCfg::CLUSTER) * 9 * Dt * Dt * sizeof(float);
+size_t wpart_bytes(int64_t B, int n_tok, int Ds, int Dt) {
+  const int64_t M = B * n_tok;
+  const int conv_splits = grid_side(n_tok) == 24 ? conv_wgrad_splits<24>(B, kNumSMs / ConvWgradCfg<24>::CLUSTER)
+                                                  : conv_wgrad_splits<14>(B, kNumSMs / ConvWgradCfg<14>::CLUSTER);
+  const size_t conv = (size_t)conv_splits * 9 * Dt * Dt * sizeof(float);
   int splits, per;   // as the align wgrad launch below
   nt_make_splits((int)((M + AlignWgradCfg::KROWS - 1) / AlignWgradCfg::KROWS), kNumSMs / (Dt / 128), &splits, &per);
   const size_t align = (size_t)splits * nt_slot_floats((int64_t)Dt * Ds) * sizeof(float), colsum = colsum_planes_part_bytes(Dt);
   const size_t m = conv > align ? conv : align;
   return m > colsum ? m : colsum;
 }
-Workspace carve(void* base, int64_t M, int Ds, int Dt, int P, bool det) {
+Workspace carve(void* base, int64_t B, int n_tok, int Ds, int Dt, int P, bool det) {
   Workspace w;
+  const int64_t M = B * n_tok;
   size_t off = 0;
   auto take = [&](size_t n) { size_t o = off; off = align_up(off + n, 1024); return reinterpret_cast<char*>(base) + o; };
   const size_t act = (size_t)P * M * Dt * 2, cw = (size_t)P * Dt * Dt * 9 * 2;
@@ -70,7 +83,7 @@ Workspace carve(void* base, int64_t M, int Ds, int Dt, int P, bool det) {
   w.dW1t = reinterpret_cast<float*>(take((size_t)9 * Dt * Dt * 4));
   w.dW2t = reinterpret_cast<float*>(take((size_t)9 * Dt * Dt * 4));
   w.partials = reinterpret_cast<double*>(take((size_t)kNumSMs * sizeof(double)));
-  w.wpart = det ? reinterpret_cast<float*>(take(wpart_bytes(M, Ds, Dt))) : nullptr;
+  w.wpart = det ? reinterpret_cast<float*>(take(wpart_bytes(B, n_tok, Ds, Dt))) : nullptr;
   w.bytes = off;
   return w;
 }
@@ -83,53 +96,62 @@ int launch_tn(GemmParams<L, E>& p, cudaStream_t st, const char* what, int* grid_
   return check_launch(what);
 }
 
-// one generator convolution (forward or dgrad): out planes = epilogue(conv3x3(in planes; w planes))
-template <int MODE>
-int run_conv(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParams ep, int64_t B, int C, int P, cudaStream_t st,
-             const char* what, int* grid_out = nullptr) {
-  using Cfg = ConvCfg;
-  using L = ConvRowsLoader<Cfg>;
+// one generator convolution (forward or dgrad) on the HW x HW grid: out planes = epilogue(conv3x3(in planes; w planes))
+template <int HW, int MODE>
+int run_conv_grid(const __nv_bfloat16* in, const __nv_bfloat16* wplanes, ConvEpiParams ep, int64_t B, int C, int P, cudaStream_t st,
+                  const char* what, int* grid_out) {
+  using Cfg = ConvCfg<HW>;
+  using L = ConvRowsLoader<Cfg, HW>;
   using E = ConvEpi<Cfg, MODE>;
   GemmParams<L, E> p;
-  int rc = make_image_tmap(&p.ld.tmX, in, B, C, P, what);
+  int rc = make_image_tmap(&p.ld.tmX, in, B, HW, C, P, what);
   if (rc != DKD_OK) return rc;
   rc = make_plane_tmap(&p.ld.tmW, wplanes, P, C, 9 * C, 9 * C, (int64_t)C * 9 * C, L::W_ROWS, what);
   if (rc != DKD_OK) return rc;
-  p.ld.total_hrows = (int)(B * kHW);
+  p.ld.total_hrows = (int)(B * HW);
   p.ld.nterms = P == 2 ? 3 : 1;
   p.ep = ep;
   p.m_tiles = (p.ld.total_hrows + L::ROWS - 1) / L::ROWS;
   p.n_tiles = 1;
   return launch_tn<Cfg, L, E>(p, st, what, grid_out);
 }
+template <int MODE>
+int run_conv(int hw, const __nv_bfloat16* in, const __nv_bfloat16* wplanes, const ConvEpiParams& ep, int64_t B, int C, int P, cudaStream_t st,
+             const char* what, int* grid_out = nullptr) {
+  return hw == 24 ? run_conv_grid<24, MODE>(in, wplanes, ep, B, C, P, st, what, grid_out)
+                  : run_conv_grid<14, MODE>(in, wplanes, ep, B, C, P, st, what, grid_out);
+}
 
 // Items = (tap, ci half) x row splits over the clusters.  The split count is chosen so that the items fill whole waves of
 // `slots` clusters: the former fixed 6 splits gave 324 items on 148 CTAs = 2.19 waves, i.e. a makespan of 3 waves for 2.19
 // waves of work (27 % idle).
+template <int HW>
 int conv_wgrad_splits(int64_t B, int slots) {
-  return nt_best_splits(NtConvLoader<ConvWgradCfg>::COMBOS_CLUSTER, slots, (int)((B * kHW + 7) / 8), 4, 16);
+  constexpr int rb = conv_wgrad_rows<HW>();
+  return nt_best_splits(NtConvLoader<ConvWgradCfg<HW>, HW>::COMBOS_CLUSTER, slots, (int)((B * HW + rb - 1) / rb), 4, 16);
 }
 
 // dW[co][ci][tap] (PyTorch layout) = sum_m G[m, co] * X[m + shift(tap), ci], through dWt[split][tap][co][ci].  `part` null:
 // the splits add into dWt with float atomics; else (deterministic mode) the split count depends on B alone and each split
 // stores its own slot of `part`, which the transpose kernel folds in split order
-int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, float* part, float* dW, int64_t B, int64_t M, int C, int P,
-                   cudaStream_t st, const char* what) {
-  using Cfg = ConvWgradCfg;
-  using L = NtConvLoader<Cfg>;
+template <int HW>
+int run_conv_wgrad_grid(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, float* part, float* dW, int64_t B, int64_t M, int C,
+                        int P, cudaStream_t st, const char* what) {
+  using Cfg = ConvWgradCfg<HW>;
+  using L = NtConvLoader<Cfg, HW>;
   GemmNtParamsT<Cfg, L> p;
   int rc = make_plane_tmap(&p.ld.tmG, G, P, M, C, C, M * C, Cfg::KROWS, what);
   if (rc != DKD_OK) return rc;
-  rc = make_image_tmap(&p.ld.tmX, X, B, C, P, what);
+  rc = make_image_tmap(&p.ld.tmX, X, B, HW, C, P, what);
   if (rc != DKD_OK) return rc;
-  p.ld.total_hrows = (int)(B * kHW);
-  p.ld.total_row_blocks = (p.ld.total_hrows + 7) / 8;
+  p.ld.total_hrows = (int)(B * HW);
+  p.ld.total_row_blocks = (p.ld.total_hrows + L::RB_ROWS - 1) / L::RB_ROWS;
   static const int resident = [] {
     auto kern = gemm_nt_kernel<Cfg, L>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
     return max_resident_clusters(kern, Cfg::CLUSTER, Cfg::THREADS, Cfg::SMEM);
   }();
-  const int sp = conv_wgrad_splits(B, part ? kNumSMs / Cfg::CLUSTER : resident);
+  const int sp = conv_wgrad_splits<HW>(B, part ? kNumSMs / Cfg::CLUSTER : resident);
   nt_make_splits(p.ld.total_row_blocks, sp, &p.ld.splits, &p.ld.row_blocks_per_split);
   p.ep.ldd = C; p.ep.alpha = 1.f; p.ep.Dcol = nullptr;
   p.nterms = P == 2 ? 3 : 1;
@@ -146,6 +168,11 @@ int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, f
   if (rc != DKD_OK) return rc;
   return launch_conv_wgrad_transpose(part ? part : dWt, C, part ? p.ld.splits : 1, dW, st);
 }
+int run_conv_wgrad(int hw, const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, float* part, float* dW, int64_t B, int64_t M, int C,
+                   int P, cudaStream_t st, const char* what) {
+  return hw == 24 ? run_conv_wgrad_grid<24>(G, X, dWt, part, dW, B, M, C, P, st, what)
+                  : run_conv_wgrad_grid<14>(G, X, dWt, part, dW, B, M, C, P, st, what);
+}
 
 }  // namespace
 }  // namespace dkd
@@ -153,11 +180,11 @@ int run_conv_wgrad(const __nv_bfloat16* G, const __nv_bfloat16* X, float* dWt, f
 extern "C" {
 
 size_t dkd_masked_generation_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision) {
-  return dkd::carve(nullptr, B * n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision)).bytes;
+  return dkd::carve(nullptr, B, n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision)).bytes;
 }
 
 size_t dkd_masked_generation_hidden_offset(int64_t B, int n_tok, int Ds, int Dt, int precision) {
-  dkd::Workspace w = dkd::carve(nullptr, B * n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision));
+  dkd::Workspace w = dkd::carve(nullptr, B, n_tok, Ds, Dt, dkd::prec_planes(precision), dkd::prec_deterministic(precision));
   return (size_t)(reinterpret_cast<char*>(w.H) - static_cast<char*>(nullptr));
 }
 
@@ -173,9 +200,10 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   const char* fn = "dkd_masked_generation_fwdbwd";
   DKD_REQUIRE(dtype == DKD_F32 || dtype == DKD_BF16, DKD_E_DTYPE, "%s: dtype %d", fn, dtype);
   DKD_REQUIRE(prec_valid(precision), DKD_E_UNSUPPORTED, "%s: precision %d", fn, precision);
-  const int n_tok = kHW * kHW;
-  DKD_REQUIRE(B > 0 && s_off >= 0 && t_off >= 0 && Ts == s_off + n_tok && Tt == t_off + n_tok, DKD_E_SHAPE,
-              "%s: expects %d patch tokens (14x14 grid) after the special tokens", fn, n_tok);
+  const int n_tok = Ts - s_off, hw = grid_side(n_tok);
+  DKD_REQUIRE(B > 0 && s_off >= 0 && t_off >= 0 && hw != 0 && Tt == t_off + n_tok, DKD_E_SHAPE,
+              "%s: expects 196 (14x14 grid) or 576 (24x24 grid) patch tokens after the special tokens in both student and teacher, "
+              "got %d and %d", fn, n_tok, Tt - t_off);
   DKD_REQUIRE(Ds == 192 && Dt == 384, DKD_E_SHAPE, "%s: built for widths 192 -> 384, got %d -> %d", fn, Ds, Dt);
   DKD_REQUIRE(s && t && mask && W_align && mask_token && conv1_w && conv1_b && conv2_w && conv2_b && loss && workspace, DKD_E_SHAPE,
               "%s: null pointer", fn);
@@ -184,7 +212,7 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   const int P = prec_planes(precision);
   const int64_t M = B * n_tok;
   DKD_REQUIRE(M < (1ll << 31) - 256, DKD_E_SHAPE, "%s: too many rows", fn);
-  Workspace ws = carve(workspace, M, Ds, Dt, P, prec_deterministic(precision));
+  Workspace ws = carve(workspace, B, n_tok, Ds, Dt, P, prec_deterministic(precision));
   DKD_REQUIRE(workspace_bytes >= ws.bytes, DKD_E_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, ws.bytes);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const bool want_grads = g_s || g_W_align || g_b_align || g_mask_token || g_conv1_w || g_conv1_b || g_conv2_w || g_conv2_b;
@@ -223,11 +251,11 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   // ---- h = relu(conv1(x_m)), g = conv2(h), masked MSE
   {
     ConvEpiParams e1 = ep; e1.out = ws.H; e1.bias = conv1_b;
-    rc = run_conv<EPI_RELU>(ws.X, ws.W1c, e1, B, Dt, P, st, "mgd: conv1");
+    rc = run_conv<EPI_RELU>(hw, ws.X, ws.W1c, e1, B, Dt, P, st, "mgd: conv1");
     if (rc != DKD_OK) return rc;
     ConvEpiParams e2 = ep; e2.out = ws.G; e2.bias = conv2_b;
     int grid = 0;
-    rc = run_conv<EPI_MSE>(ws.H, ws.W2c, e2, B, Dt, P, st, "mgd: conv2", &grid);
+    rc = run_conv<EPI_MSE>(hw, ws.H, ws.W2c, e2, B, Dt, P, st, "mgd: conv2", &grid);
     if (rc != DKD_OK) return rc;
     rc = launch_fold_partials(ws.partials, grid, scale, loss, st);
     if (rc != DKD_OK) return rc;
@@ -236,7 +264,7 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
 
   // ---- conv2 backward
   if (g_conv2_w) {
-    rc = run_conv_wgrad(ws.G, ws.H, ws.dW2t, ws.wpart, g_conv2_w, B, M, Dt, P, st, "mgd: conv2 wgrad");
+    rc = run_conv_wgrad(hw, ws.G, ws.H, ws.dW2t, ws.wpart, g_conv2_w, B, M, Dt, P, st, "mgd: conv2 wgrad");
     if (rc != DKD_OK) return rc;
   }
   if (g_conv2_b) {
@@ -245,12 +273,12 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   }
   {
     ConvEpiParams e = ep; e.out = ws.DH; e.act = ws.H;
-    rc = run_conv<EPI_DRELU>(ws.G, ws.W2d, e, B, Dt, P, st, "mgd: conv2 dgrad");
+    rc = run_conv<EPI_DRELU>(hw, ws.G, ws.W2d, e, B, Dt, P, st, "mgd: conv2 dgrad");
     if (rc != DKD_OK) return rc;
   }
   // ---- conv1 backward
   if (g_conv1_w) {
-    rc = run_conv_wgrad(ws.DH, ws.X, ws.dW1t, ws.wpart, g_conv1_w, B, M, Dt, P, st, "mgd: conv1 wgrad");
+    rc = run_conv_wgrad(hw, ws.DH, ws.X, ws.dW1t, ws.wpart, g_conv1_w, B, M, Dt, P, st, "mgd: conv1 wgrad");
     if (rc != DKD_OK) return rc;
   }
   if (g_conv1_b) {
@@ -260,7 +288,7 @@ int dkd_masked_generation_fwdbwd(const void* s, const void* t, const float* mask
   if (!(g_s || g_W_align || g_b_align || g_mask_token)) return DKD_OK;
   {
     ConvEpiParams e = ep; e.out = ws.G;  // dXm overwrites G (no longer needed)
-    rc = run_conv<EPI_PLAIN>(ws.DH, ws.W1d, e, B, Dt, P, st, "mgd: conv1 dgrad");
+    rc = run_conv<EPI_PLAIN>(hw, ws.DH, ws.W1d, e, B, Dt, P, st, "mgd: conv1 dgrad");
     if (rc != DKD_OK) return rc;
   }
   // ---- mask-token / alignment backward: masked rows feed mask_token, kept rows feed the Linear

@@ -145,12 +145,13 @@ _ZOO = {
 }
 
 
-def create_model(name: str, num_classes: int = 1000, row_ops: str = "aten", **_) -> DeiT:
-    """Stand-in for timm.create_model(name, pretrained=False, num_classes=...) restricted to the DeiT variants the
-    reference's exp/*.sh scripts use, plus the DeiT-Base teacher.  `row_ops="dkd"` builds the same model (same state_dict) on libdeltakd_sm100's
+def create_model(name: str, num_classes: int = 1000, row_ops: str = "aten", img_size: int = 224, **_) -> DeiT:
+    """Stand-in for timm.create_model(name, pretrained=False, num_classes=..., img_size=...) restricted to the DeiT variants the
+    reference's exp/*.sh scripts use, plus the DeiT-Base teacher.  `img_size` is timm's keyword: 384 gives the 24 x 24 patch
+    grid of the DeiT "384" recipe (577 tokens, 578 distilled).  `row_ops="dkd"` builds the same model (same state_dict) on libdeltakd_sm100's
     LayerNorm / bias-gradient / head-relayout kernels — CUDA only."""
     if name not in _ZOO:
         raise ValueError(f"unknown model {name}; available: {sorted(_ZOO)}")
     if row_ops not in _ROW_OPS:
         raise ValueError(f"row_ops must be one of {sorted(_ROW_OPS)}, got {row_ops!r}")
-    return DeiT(num_classes=num_classes, row_ops=row_ops, **_ZOO[name])
+    return DeiT(num_classes=num_classes, row_ops=row_ops, img_size=img_size, **_ZOO[name])

@@ -362,15 +362,22 @@ SUPPORTED_PAIRS = {
     "masked generation": (_DEIT_TS,),
     "LRKD": (_DEIT_TS,),
 }
-SUPPORTED_GRID_TOKENS = 196       # 14 x 14 patch grid (224-px inputs, patch 16) for the generator conv / Sinkhorn kernels
+# patch-token counts (square grids, patch 16) of the entry points whose kernels are built for given grids: the generator
+# convolutions and the Sinkhorn cost matrix.  Every other entry point takes any token count.
+_GRID_NAMES = {196: "14 x 14 grid: 224-px inputs", 576: "24 x 24 grid: 384-px inputs"}
+SUPPORTED_GRID_TOKENS = {
+    "masked generation": (196, 576),
+    "dkd_wass_sinkhorn": (196,),
+}
 
 
-def _check_feature_pair(s, t, s_off, t_off, op: str, grid_tokens: bool = False):
+def _check_feature_pair(s, t, s_off, t_off, op: str):
     """Validates one (student, teacher) feature pair for the entry point `op` (a key of SUPPORTED_PAIRS) and states the
     pairs it supports in the error: every feature loss is built for DeiT-Tiny -> DeiT-Small widths (192 -> 384), which
     is what all 19 exp/*.sh scripts of the reference use, and the hidden-state matching and WassKD-l1 losses also for a
-    DeiT-Base teacher (192 -> 768); other timm pairs (e.g. a 384-wide student, 384-px inputs) are rejected here, at the
-    first call, instead of failing deep inside a launch."""
+    DeiT-Base teacher (192 -> 768).  Masked generation and Sinkhorn also check the patch-token count against
+    SUPPORTED_GRID_TOKENS.  Other timm pairs (e.g. a 384-wide student) and grids are rejected here, at the first call,
+    instead of failing deep inside a launch."""
     _require_cuda(s, t)
     if s.dim() != 3 or t.dim() != 3 or s.shape[0] != t.shape[0]:
         raise ValueError(f"features must be [B, tokens, dim]; got {tuple(s.shape)} and {tuple(t.shape)}")
@@ -381,9 +388,11 @@ def _check_feature_pair(s, t, s_off, t_off, op: str, grid_tokens: bool = False):
         built = " and ".join(f"{ds} -> {dt} ({_PAIR_NAMES[(ds, dt)]})" for ds, dt in pairs)
         raise ValueError(f"deltakd_b200 {op}: built for student/teacher widths {built}; got {s.shape[2]} -> {t.shape[2]}. "
                          "See INTEGRATION.md 'Supported model matrix'.")
-    if grid_tokens and s.shape[1] - s_off != SUPPORTED_GRID_TOKENS:
-        raise ValueError(f"deltakd_b200 {op}: built for {SUPPORTED_GRID_TOKENS} patch tokens (14 x 14 grid: 224-px inputs, patch 16); "
-                         f"got {s.shape[1] - s_off}. See INTEGRATION.md 'Supported model matrix'.")
+    grids = SUPPORTED_GRID_TOKENS.get(op)
+    if grids is not None and s.shape[1] - s_off not in grids:
+        built = " or ".join(f"{n} patch tokens ({_GRID_NAMES[n]}, patch 16)" for n in grids)
+        raise ValueError(f"deltakd_b200 {op}: built for {built}; got {s.shape[1] - s_off}. "
+                         "See INTEGRATION.md 'Supported model matrix'.")
 
 
 def align_mse_layers_loss(s_feats, t_feats, linears, scale: float, s_off: int = 1, t_off: int = 2,
@@ -392,7 +401,7 @@ def align_mse_layers_loss(s_feats, t_feats, linears, scale: float, s_off: int = 
     n = len(linears)
     s_list, t_list, w_list, b_list = [], [], [], []
     for s, t, lin in zip(_f16_up_list(s_feats), _f16_up_list(t_feats), linears):
-        _check_feature_pair(s, t, s_off, t_off, op=_entry, grid_tokens=_entry == "dkd_wass_sinkhorn")
+        _check_feature_pair(s, t, s_off, t_off, op=_entry)
         t = t.detach()
         if t.dtype != s.dtype:
             t = t.to(s.dtype)
@@ -471,12 +480,14 @@ def masked_generation_loss(s_feat, t_feat, align, mask_token, generation, *, sca
                            mask_ratio=None, noise=None, s_off: int = 1, t_off: int = 2, probe: dict | None = None):
     """scale * sum(mask * (generation(where(mask, mask_token, align(s[:, s_off:]))) - t[:, t_off:])**2).
 
-    `mask` [B,196] (1 = masked) is used if given; otherwise it is drawn like the reference's
-    random_masking: noise = torch.rand(B, 196, device) (misc.py:14) -> rank -> mask (dkd_mask_rank).
+    The patch tokens form a square grid: N = 196 (14 x 14, 224-px inputs) or 576 (24 x 24, 384-px inputs), the same N
+    for student and teacher (SUPPORTED_GRID_TOKENS).
+    `mask` [B,N] (1 = masked) is used if given; otherwise it is drawn like the reference's
+    random_masking: noise = torch.rand(B, N, device) (misc.py:14) -> rank -> mask (dkd_mask_rank).
     `probe` (verification only): receives "mask" and "hidden" = the generator's post-ReLU activations as bf16 planes
-    [P, B, 196, Dt], i.e. the ReLU gate the fused backward used (tests compare gradients given that gate)."""
+    [P, B, N, Dt], i.e. the ReLU gate the fused backward used (tests compare gradients given that gate)."""
     s_feat, t_feat = _f16_up(s_feat), _f16_up(t_feat)
-    _check_feature_pair(s_feat, t_feat, s_off, t_off, op="masked generation", grid_tokens=True)
+    _check_feature_pair(s_feat, t_feat, s_off, t_off, op="masked generation")
     B = s_feat.shape[0]
     L = s_feat.shape[1] - s_off
     if mask is None:

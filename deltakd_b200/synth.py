@@ -46,18 +46,18 @@ def make_logits(B: int, C: int, seed: int = 1234, int_labels: bool = False):
 
 
 def make_features(B: int, seed: int = 1234, layers=range(NUM_LAYERS), scale: float = 1.0, t_shift: float = 0.0,
-                  teacher_dim: int = TEACHER_DIM):
-    """12-entry lists (None where the layer is not requested) of student [B,197,192] and
-    teacher [B,198,teacher_dim] fp32 tensors (384: DeiT-Small, 768: DeiT-Base).  `scale`/`t_shift` give the
-    Sinkhorn variant of §8d."""
+                  teacher_dim: int = TEACHER_DIM, n_tok: int = STUDENT_TOKENS - 1):
+    """12-entry lists (None where the layer is not requested) of student [B,1+n_tok,192] and
+    teacher [B,2+n_tok,teacher_dim] fp32 tensors (384: DeiT-Small, 768: DeiT-Base).  `n_tok` is the patch-token count:
+    196 for 224-px inputs, 576 for 384-px inputs.  `scale`/`t_shift` give the Sinkhorn variant of §8d."""
     layers = set(int(i) % NUM_LAYERS for i in layers)
     s_feats, t_feats = [None] * NUM_LAYERS, [None] * NUM_LAYERS
     for i in range(NUM_LAYERS):
         if i not in layers:
             continue
         g = _gen(seed * 1000 + i)
-        s_feats[i] = torch.randn(B, STUDENT_TOKENS, STUDENT_DIM, generator=g) * scale
-        t_feats[i] = torch.randn(B, TEACHER_TOKENS, teacher_dim, generator=g) * scale + t_shift
+        s_feats[i] = torch.randn(B, 1 + n_tok, STUDENT_DIM, generator=g) * scale
+        t_feats[i] = torch.randn(B, 2 + n_tok, teacher_dim, generator=g) * scale + t_shift
     return s_feats, t_feats
 
 

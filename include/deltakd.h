@@ -194,21 +194,23 @@ DKD_API int dkd_wass_sinkhorn_fwdbwd(const void* s, const void* t, const float* 
                                      size_t workspace_bytes, dkd_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Masked generative distillation core, forward + backward (14x14 token grid, Ds = 192, Dt = 384):
+ * Masked generative distillation core, forward + backward (Ds = 192, Dt = 384) on a square patch grid of
+ * n_tok = Ts - s_off = Tt - t_off tokens: 196 (14x14, 224-px inputs, patch 16) or 576 (24x24, 384-px inputs); any
+ * other count returns DKD_E_SHAPE:
  *     x   = s[:, s_off:, :] W_align^T + b_align
  *     x_m = where(mask, mask_token, x)
  *     g   = conv3x3(relu(conv3x3(x_m; conv1)); conv2)          (pad 1, NHWC = the token layout)
  *     *loss += scale * sum( mask * (g - t[:, t_off:, :])^2 )   (accumulates)
  * plus the gradients of every input that has a non-NULL g_* pointer (all overwritten).
- * Replaces mgd_loss (model/loss.py:422-451; scale = mgd_alpha/(B*196*Dt)), saliency_mgd_loss (:335-360;
- * scale = 4/(B*196*Dt)), the late phase of curkd_loss (:394-420; scale = 5e-5/B) and the ViTKD
+ * Replaces mgd_loss (model/loss.py:422-451; scale = mgd_alpha/(B*n_tok*Dt)), saliency_mgd_loss (:335-360;
+ * scale = 4/(B*n_tok*Dt)), the late phase of curkd_loss (:394-420; scale = 5e-5/B) and the ViTKD
  * generation term (:291-310), including `student.generation` = Conv2d-ReLU-Conv2d (models.py:148-151).
- *   mask : fp32 [B, 196], 1 = masked (from dkd_mask_rank) ;  mask_token : fp32 [Dt]
+ *   mask : fp32 [B, n_tok], 1 = masked (from dkd_mask_rank) ;  mask_token : fp32 [Dt]
  *   conv*_w : fp32 [Dt, Dt, 3, 3] (PyTorch layout), conv*_b : fp32 [Dt]
  */
 DKD_API size_t dkd_masked_generation_workspace_bytes(int64_t B, int n_tok, int Ds, int Dt, int precision);
 /* Byte offset, inside the workspace, of the generator's hidden activations h = relu(conv1(x_m)) as bf16 planes
- * [P][B*196][Dt] (P = 2 hi/lo planes for DKD_PREC_BF16X3, else 1; DKD_PREC_DETERMINISTIC does not move them).  They
+ * [P][B*n_tok][Dt] (P = 2 hi/lo planes for DKD_PREC_BF16X3, else 1; DKD_PREC_DETERMINISTIC does not move them).  They
  * stay valid after dkd_masked_generation_fwdbwd
  * returns: verification code reads the ReLU gate the backward pass used from them (h != 0), because the gradient of
  * F.relu (models.py:150) is discontinuous at 0 and parity of the gradients is only defined given the same gate. */
